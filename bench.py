@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the i-DQN learning step (BASELINE.json metric: gradient steps/s, NatureCNN K=5, batch 32).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Ours, N GPUs: one process per GPU (torchrun for N>1); each rank owns 5 heads of one 5N-head i-DQN chain
 (weak scaling, head-sharded; the only cross-GPU traffic is the neighbour target exchange every D / T steps, a kernel
@@ -188,6 +188,31 @@ def source_sha() -> str:
     return h.hexdigest()[:16]
 
 
+DUMP_SAMPLE = 65536  # entries kept per head of a larger leaf (only Dense_0/kernel, 3.96 M per head, at the bench sizes)
+
+
+def dump_outputs(agent, L, out_dir):
+    """Writes what the timed resident path leaves its caller after its last step, one DIR/<name>.npy per array: the
+    online and target parameters, the Adam moments and step counts, the device-side loss sums (idqn.py:63,72) and the
+    |TD| of the last step per head and sample.  A leaf larger than DUMP_SAMPLE entries per head is reduced to a fixed,
+    seeded sample of its entries, the same ones in every tree: about 12 MB in all at K = 5."""
+    eng = agent._engine
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"cumulated_losses": agent.cumulated_losses, "td_abs": eng.td_abs(),
+           "optimizer_state.count": eng.get_count().astype(np.float64)}
+    for i, info in enumerate(eng.leaves):
+        pick = None
+        if info["size"] > DUMP_SAMPLE:
+            pick = np.sort(np.random.default_rng(i).choice(info["size"], DUMP_SAMPLE, replace=False))
+        leaf = info["module"].replace("/", ".") + "." + info["kind"]
+        for tree, which in (("params", L.ONLINE), ("target_params", L.TARGET), ("optimizer_state.mu", L.MU),
+                            ("optimizer_state.nu", L.NU)):
+            a = eng.download_leaf(which, i)
+            out[f"{tree}.{leaf}"] = a if pick is None else a.reshape(eng.K, -1)[:, pick]
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -281,6 +306,8 @@ def run_ours(args):
 
     ms, wall, clocks, nxt = timed(eng, resident_step, args.steps, args.warmup, 1, clocks=True)
     steps_per_s = args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(agent, L, args.dump_outputs)
 
     # (2) end to end through the host-buffer C-ABI call: pinned host batch -> H2D -> step -> D2H losses
     pool = []
@@ -710,7 +737,12 @@ def main():
     ap.add_argument("--no-prioritized", action="store_true", help="skip the prioritised-replay (configs[4]) leg")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the us/step figures of configs[0..2]")
     ap.add_argument("--flags", type=int, default=0, help="IDQN_F_* engine flags (A/B experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the state the resident path computed as DIR/<name>.npy "
+                         "(rank 0's heads), to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
