@@ -95,6 +95,10 @@ SYMBOLS = {
     "idqn_replay_put": (_I, [_P, _I64, _P, _P, C.c_int32, C.c_double, C.c_uint8, C.c_uint8]),
     "idqn_replay_gather_host": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _P]),
     "idqn_learn_from_replay": (_I, [_P, _P, _P, _I, _I, _P]),
+    "idqn_replay_create_frames": (_I, [_I64, _I64, _I, _I, _I64, _I, C.POINTER(_P)]),
+    "idqn_replay_put_frame": (_I, [_P, _I64, _P]),
+    "idqn_replay_put_element": (_I, [_P, _I64, _P, C.c_int32, C.c_double, C.c_uint8, C.c_uint8]),
+    "idqn_replay_grow_frames": (_I, [_P, _I64, _I64, _I64]),
 }
 
 _lock = threading.Lock()

@@ -7,6 +7,7 @@
 #include <stdio.h>
 #include <stdarg.h>
 #include <string.h>
+#include <unordered_set>
 #include <vector>
 
 #include "../../include/idqn_b200.h"
@@ -110,6 +111,13 @@ struct FastDiv {
     r = n - q * d;
   }
 };
+
+// ring slot of frame id `id` (>= 0) in a frame store of n_frames frames: 32-bit remainder while both fit (every id of a
+// run shorter than 2^32 frames), the 64-bit one after
+__host__ __device__ __forceinline__ int64_t frame_ring_slot(int64_t id, int64_t n_frames) {
+  if ((((uint64_t)id | (uint64_t)n_frames) >> 32) == 0) return (int64_t)((uint32_t)id % (uint32_t)n_frames);
+  return id % n_frames;
+}
 
 // ---------------------------------------------------------------------------------------------
 // One layer of DQNNet seen as a convolution (Dense == 1x1 conv on a 1x1 image with IC = fan-in).
@@ -246,6 +254,12 @@ struct idqn_handle {
     const int32_t* action;
     const double* reward;
     const uint8_t* terminal;
+    // frame store (idqn_replay_create_frames): state/next_state are null and image g of slot s is assembled from the
+    // frames rows[(s * 2 + g) * stack + c] (id -1: a zero frame), frame id f at ring + (f % n_frames) * frame_bytes
+    const uint8_t* ring;
+    const int64_t* rows;
+    int64_t n_frames, frame_bytes;
+    int stack;
   } rsrc;
   int rsrc_on;
   int graph_set;             // staging set the next step reads (idqn_submit_batch_host points the step at its slot)
@@ -276,6 +290,17 @@ struct idqn_replay {
   cudaEvent_t ev_learner;
   int learner_pending;
   std::vector<int64_t>* learner_slots;
+  // frame store (idqn_replay_create_frames; state/next_state stay null): each observation once, in a ring of n_frames
+  // frames of value_bytes-byte values; slot s holds 2*stack frame ids (state positions, then next_state positions; -1 = zero frame) in rows and its
+  // host mirror h_rows.  state_bytes = frame_bytes * stack.  Unlike learner_slots, the element rows and ring slots of
+  // the in-flight steps accumulate until ev_learner has completed: a write into any of them waits for it.
+  int frames;
+  int stack, value_bytes;
+  int64_t frame_bytes, n_frames;
+  uint8_t* ring;
+  int64_t* rows;
+  int64_t* h_rows;
+  std::unordered_set<int64_t> *inflight_rows, *inflight_frames;
   // pinned staging for gather_host
   void* h_stage;
   size_t h_stage_bytes;

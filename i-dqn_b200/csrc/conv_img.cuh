@@ -1068,6 +1068,12 @@ struct S2dArgs {
   const int32_t* g_action;
   const double* g_reward;
   const uint8_t* g_terminal;
+  // ring != nullptr (with slots): frame store -- src is unused and value v * stack + p of image g of slot s is value v of
+  // frame rows[(s * 2 + g) * stack + p] (id -1: zero), frame id f at ring + (f % n_frames) * frame_bytes
+  const uint8_t* ring;
+  const int64_t* rows;
+  int64_t n_frames, frame_bytes;
+  int stack;
   int32_t* o_action;
   float* o_reward;
   uint8_t* o_terminal;
@@ -1077,6 +1083,8 @@ struct S2dArgs {
   bf16 *hi, *lo;       // [2][imgs][img_rows][C2]
   int tl_id;
 };
+// kFrames: the frame-store source (a.ring); a separate instance, so the element paths compile exactly as without it
+template <bool kFrames>
 __global__ void __launch_bounds__(256) s2d_input_kernel(const S2dArgs a) {
   // one thread per (g, img, by, bx, ry): s*IC contiguous output channels = s input pixels of one input row
   pdl_trigger();
@@ -1102,18 +1110,43 @@ __global__ void __launch_bounds__(256) s2d_input_kernel(const S2dArgs a) {
     const int im = (int)(t % a.imgs), g = (int)(t / a.imgs);
     const int iy = by * a.s + ry - a.ph;
     const int64_t o = (((int64_t)g * a.imgs + im) * a.img_rows + (int64_t)by * a.P + bx) * a.C2 + (int64_t)ry * run;
-    if (a.u8 && a.IC == 4 && a.s == 4 && (a.pw & 1) == 0 && (a.IW & 1) == 0) {
+    if (a.u8 && a.IC == 4 && a.s == 4 && (a.pw & 1) == 0 && (a.IW & 1) == 0 && (!kFrames || a.stack == 4)) {
       // Atari frames: the run is 4 pixels x 4 stacked frames = 16 source bytes, 8-byte aligned pixel pairs
-      const uint8_t* src = (const uint8_t*)(g ? a.src[1] : a.src[0]) + (a.slots ? a.slots[im] * a.src_stride : (int64_t)im * img_elems);
       const int ix0 = bx * 4 - a.pw;
-      uint2 raw[2];
+      uint32_t w[4];  // w[q]: the 4 stacked frames of pixel ix0 + q, frame c in byte c
+      if constexpr (kFrames) {
+        // frame store: the same 16 bytes from the 4 frames, a 2-byte aligned pixel pair of each (ix0 is even, not a
+        // multiple of 4), interleaved pixel-major
+        const int64_t* row = a.rows + (a.slots[im] * 2 + g) * 4;
+        const uint8_t* f[4];
 #pragma unroll
-      for (int hp = 0; hp < 2; ++hp) {
-        const int ix = ix0 + 2 * hp;
-        const bool ok = (unsigned)iy < (unsigned)a.IH && ix >= 0 && ix + 1 < a.IW;
-        raw[hp] = ok ? __ldg(reinterpret_cast<const uint2*>(src + ((int64_t)iy * a.IW + ix) * 4)) : make_uint2(0, 0);
+        for (int c = 0; c < 4; ++c) {
+          const int64_t id = __ldg(row + c);
+          f[c] = id < 0 ? nullptr : a.ring + frame_ring_slot(id, a.n_frames) * a.frame_bytes;
+        }
+#pragma unroll
+        for (int hp = 0; hp < 2; ++hp) {
+          const int ix = ix0 + 2 * hp;
+          const bool ok = (unsigned)iy < (unsigned)a.IH && ix >= 0 && ix + 1 < a.IW;
+          uint32_t p[4];
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+            p[c] = ok && f[c] ? __ldg(reinterpret_cast<const unsigned short*>(f[c] + (int64_t)iy * a.IW + ix)) : 0u;
+          const uint32_t p01 = p[0] | (p[1] << 16), p23 = p[2] | (p[3] << 16);
+          w[2 * hp] = __byte_perm(p01, p23, 0x6420);      // first pixel of the pair, frames 0..3
+          w[2 * hp + 1] = __byte_perm(p01, p23, 0x7531);  // second pixel
+        }
+      } else {
+        const uint8_t* src = (const uint8_t*)(g ? a.src[1] : a.src[0]) + (a.slots ? a.slots[im] * a.src_stride : (int64_t)im * img_elems);
+        uint2 raw[2];
+#pragma unroll
+        for (int hp = 0; hp < 2; ++hp) {
+          const int ix = ix0 + 2 * hp;
+          const bool ok = (unsigned)iy < (unsigned)a.IH && ix >= 0 && ix + 1 < a.IW;
+          raw[hp] = ok ? __ldg(reinterpret_cast<const uint2*>(src + ((int64_t)iy * a.IW + ix) * 4)) : make_uint2(0, 0);
+        }
+        w[0] = raw[0].x, w[1] = raw[0].y, w[2] = raw[1].x, w[3] = raw[1].y;
       }
-      const uint32_t w[4] = {raw[0].x, raw[0].y, raw[1].x, raw[1].y};
 #pragma unroll
       for (int hv = 0; hv < 2; ++hv) {
         float x[8];
@@ -1133,8 +1166,13 @@ __global__ void __launch_bounds__(256) s2d_input_kernel(const S2dArgs a) {
         if ((unsigned)iy < (unsigned)a.IH && (unsigned)ix < (unsigned)a.IW) {
           const int64_t si = ((int64_t)iy * a.IW + ix) * a.IC + c;
           const void* src = g ? a.src[1] : a.src[0];
-          if (a.slots) v = (float)__ldg((const uint8_t*)src + a.slots[im] * a.src_stride + si);  // replay slots hold uint8 frames here
-          else v = a.u8 ? (float)__ldg((const uint8_t*)src + (int64_t)im * img_elems + si) : __ldg((const float*)src + (int64_t)im * img_elems + si);
+          if constexpr (kFrames) {
+            const int64_t id = __ldg(a.rows + (a.slots[im] * 2 + g) * a.stack + si % a.stack);
+            if (id >= 0) v = (float)__ldg(a.ring + frame_ring_slot(id, a.n_frames) * a.frame_bytes + si / a.stack);
+          } else {
+            if (a.slots) v = (float)__ldg((const uint8_t*)src + a.slots[im] * a.src_stride + si);  // replay slots hold uint8 frames here
+            else v = a.u8 ? (float)__ldg((const uint8_t*)src + (int64_t)im * img_elems + si) : __ldg((const float*)src + (int64_t)im * img_elems + si);
+          }
         }
         x[k] = v;
       }

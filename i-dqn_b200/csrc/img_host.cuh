@@ -503,10 +503,12 @@ static int img_launch_s2d(idqn_handle* h, int x_u8, bool single_state = false) {
   a.tl_id = single_state ? -1 : tl_next(h);
   if (single_state) a.imgs = 1, a.n_src = 1;
   a.src[0] = h->s, a.src[1] = h->s2;  // the staging set of this step (idqn_submit_batch_host points it at its slot)
-  a.slots = nullptr;
+  a.slots = nullptr, a.ring = nullptr;
   if (h->rsrc_on) {  // idqn_learn_from_replay: frames read from the replay slots in place, scalars gathered here
     a.src[0] = h->rsrc.state, a.src[1] = h->rsrc.next_state;
     a.slots = h->rsrc.slots, a.src_stride = h->rsrc.state_bytes;
+    a.ring = h->rsrc.ring, a.rows = h->rsrc.rows, a.n_frames = h->rsrc.n_frames, a.frame_bytes = h->rsrc.frame_bytes;
+    a.stack = h->rsrc.stack;
     a.g_action = h->rsrc.action, a.g_reward = h->rsrc.reward, a.g_terminal = h->rsrc.terminal;
     a.o_action = h->action, a.o_reward = h->reward, a.o_terminal = h->terminal;
   }
@@ -514,7 +516,9 @@ static int img_launch_s2d(idqn_handle* h, int x_u8, bool single_state = false) {
   // first kernel of the step: launched WITHOUT the programmatic attribute, so everything enqueued before the step (the
   // previous step's Adam kernels when the step is not graph-replayed) has completed before any kernel of this step --
   // several of which prefetch weight tiles ahead of their griddepcontrol.wait -- can start
-  CK(launch_pdl(false, img::s2d_input_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, h->stream, a));
+  const dim3 grid((unsigned)((total + 255) / 256));
+  if (a.ring) CK(launch_pdl(false, img::s2d_input_kernel<true>, grid, dim3(256), 0, h->stream, a));
+  else CK(launch_pdl(false, img::s2d_input_kernel<false>, grid, dim3(256), 0, h->stream, a));
   mark(h, "s2d_input_L%d", 0);
   return IDQN_OK;
 }

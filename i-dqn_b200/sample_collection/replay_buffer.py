@@ -8,7 +8,12 @@ gather kernel writing straight into the learner's batch staging (``learn_step_on
 dict-lookup + decompress + np.stack + H2D path of the reference disappears.
 
 FIFO semantics are the reference's: keys are the cumulative ``add_count`` (:207), the oldest key is evicted
-once ``add_count > max_capacity`` (:211-213); key ``k`` lives in slot ``k % max_capacity``."""
+once ``add_count > max_capacity`` (:211-213); key ``k`` lives in slot ``k % max_capacity``.
+
+``frame_store=True`` keeps each observation once (the memory saving the reference gets from ``compress=True``,
+:36-57,204-205): a device ring of frames plus, per element, the frame ids of its two stacks.  The host side of it
+(which frames exist, when the ring must grow) is plain bookkeeping over a store object with ``put_frame`` /
+``put_element`` / ``grow``."""
 from __future__ import annotations
 
 import collections
@@ -98,6 +103,44 @@ class _DeviceStore:
         return s, s2, a.astype(np.int64), r, d.astype(bool), e.astype(bool)
 
 
+class _FrameStore:
+    """Frame store in HBM (idqn_replay_create_frames): a ring of ``n_frames`` observations (frame id ``f`` in ring slot
+    ``f % n_frames``) and, per element slot, ``2 * stack`` frame ids (-1: a zero frame)."""
+
+    def __init__(self, n_slots: int, frame_shape, frame_dtype, stack: int, n_frames: int, device: int):
+        self.lib = L.lib()
+        self.frame_shape, self.dtype, self.stack = tuple(frame_shape), np.dtype(frame_dtype), int(stack)
+        self.shape = self.frame_shape + (self.stack,)  # of a stack, as _DeviceStore.shape
+        self.frame_bytes = int(np.prod(self.frame_shape)) * self.dtype.itemsize
+        self.n_slots, self.device, self._n_frames = int(n_slots), int(device), int(n_frames)
+        h = C.c_void_p()
+        L.check(self.lib.idqn_replay_create_frames(self.n_slots, self.frame_bytes, self.stack, self.dtype.itemsize,
+                                                   self._n_frames, self.device, C.byref(h)))
+        self.h = h
+        self._finalizer = weakref.finalize(self, self.lib.idqn_replay_destroy, h)
+
+    @property
+    def n_frames(self) -> int:
+        return self._n_frames
+
+    def put_frame(self, frame_id: int, frame) -> None:
+        f = np.ascontiguousarray(frame, dtype=self.dtype)
+        if f.shape != self.frame_shape:
+            raise ValueError(f"observation shape {f.shape} differs from the store's {self.frame_shape}")
+        L.check(self.lib.idqn_replay_put_frame(self.h, int(frame_id), L.ptr(f)))
+
+    def put_element(self, slot: int, frame_ids, action, reward, is_terminal, episode_end) -> None:
+        ids = np.ascontiguousarray(frame_ids, dtype=np.int64)
+        L.check(self.lib.idqn_replay_put_element(self.h, int(slot), L.ptr(ids), int(action), float(reward),
+                                                 int(bool(is_terminal)), int(bool(episode_end))))
+
+    def grow(self, n_frames: int, live_lo: int, live_hi: int) -> None:
+        L.check(self.lib.idqn_replay_grow_frames(self.h, int(n_frames), int(live_lo), int(live_hi)))
+        self._n_frames = int(n_frames)
+
+    gather = _DeviceStore.gather
+
+
 class _MemoryView(collections.abc.Mapping):
     """``rb._memory`` of the reference (an OrderedDict key -> ReplayElement) as a read-only view of the
     device store: live keys in insertion order, elements fetched on access."""
@@ -139,6 +182,7 @@ class ReplayBuffer:
         clipping: callable = None,
         *,
         device: int = 0,
+        frame_store: bool = False,
     ):
         self.add_count = 0
         self._max_capacity = max_capacity
@@ -155,9 +199,18 @@ class ReplayBuffer:
         self._memory = _MemoryView(self)
         self._trajectory: "collections.deque[TransitionElement]" = collections.deque(
             maxlen=self._update_horizon + self._stack_size)
+        self._frame_store = frame_store
+        if frame_store:
+            # frame id of each trajectory entry once an emitted element has referred to it (None before)
+            self._frame_ids: "collections.deque[Optional[int]]" = collections.deque(maxlen=self._trajectory.maxlen)
+            self._next_frame_id = 0
+            # (key, smallest frame id) of live elements with that id increasing: the front is the smallest of all
+            self._live_min: "collections.deque[tuple[int, int]]" = collections.deque()
 
     # ---- n-step / frame-stack accumulator (replay_buffer.py:103-200) ---------------------------------
-    def _make_replay_element(self) -> Optional[ReplayElement]:
+    def _window(self) -> Optional[tuple[int, list[int]]]:
+        """The element the trajectory emits now, as (pivot, trajectory index of each of the 2 * stack stack positions:
+        state, then next_state; -1 = zero), or None."""
         traj, n, stack = self._trajectory, self._update_horizon, self._stack_size
         length = len(traj)
         newest = traj[-1]
@@ -166,42 +219,118 @@ class ReplayBuffer:
         # a terminal cuts the n-step window short when the trajectory is still shorter than n (:116-118)
         horizon = length - 1 if (newest.is_terminal and length <= n) else n
         pivot = length - horizon - 1  # newest frame of the state stack; its action is the element's action
-        frame = np.asarray(newest.observation)
-        state = np.zeros(frame.shape + (stack,), frame.dtype)  # missing history stays zero (:125,136)
+        # missing history stays zero (:125,136)
+        state = [max(pivot - (stack - 1) + pos, -1) for pos in range(stack)]
+        next_state = [max(length - stack + pos, -1) for pos in range(stack)]
+        return pivot, state + next_state
+
+    def _scalars(self, pivot: int) -> tuple[Any, float, bool]:
+        traj, n = self._trajectory, self._update_horizon
+        ret = 0.0
+        for t in range(pivot, min(pivot + n, len(traj))):  # discounted n-step return (:153-165)
+            ret += traj[t].reward * (self._gamma ** (t - pivot))
+        return traj[pivot].action, ret, traj[-1].is_terminal
+
+    def _make_replay_element(self, window) -> ReplayElement:
+        pivot, positions = window
+        traj, stack = self._trajectory, self._stack_size
+        frame = np.asarray(traj[-1].observation)
+        state = np.zeros(frame.shape + (stack,), frame.dtype)
         next_state = np.zeros(frame.shape + (stack,), frame.dtype)
         for pos in range(stack):
-            t_state, t_next = pivot - (stack - 1) + pos, length - stack + pos
+            t_state, t_next = positions[pos], positions[stack + pos]
             if t_state >= 0:
                 state[..., pos] = traj[t_state].observation
             if t_next >= 0:
                 next_state[..., pos] = traj[t_next].observation
-        ret = 0.0
-        for t in range(pivot, min(pivot + n, length)):  # discounted n-step return (:153-165)
-            ret += traj[t].reward * (self._gamma ** (t - pivot))
-        return ReplayElement(state=state, action=traj[pivot].action, reward=ret, next_state=next_state,
-                             is_terminal=newest.is_terminal, episode_end=newest.is_terminal)
+        action, ret, terminal = self._scalars(pivot)
+        return ReplayElement(state=state, action=action, reward=ret, next_state=next_state, is_terminal=terminal,
+                             episode_end=terminal)
+
+    def _windows(self, transition: TransitionElement) -> Iterator[tuple[int, list[int]]]:
+        self._trajectory.append(transition)
+        if self._frame_store:
+            self._frame_ids.append(None)
+        if transition.is_terminal:  # drain: one element per remaining start frame (:189-194)
+            while (window := self._window()) is not None:
+                yield window
+                self._trajectory.popleft()
+                if self._frame_store:
+                    self._frame_ids.popleft()
+            self._clear_trajectory()
+        else:
+            if (window := self._window()) is not None:
+                yield window
+            if transition.episode_end:  # truncation (:199-200)
+                self._clear_trajectory()
+
+    def _clear_trajectory(self) -> None:
+        self._trajectory.clear()
+        if self._frame_store:
+            self._frame_ids.clear()
 
     def accumulate(self, transition: TransitionElement) -> Iterable[ReplayElement]:
-        self._trajectory.append(transition)
-        if transition.is_terminal:  # drain: one element per remaining start frame (:189-194)
-            while (element := self._make_replay_element()) is not None:
-                yield element
-                self._trajectory.popleft()
-            self._trajectory.clear()
-        else:
-            if (element := self._make_replay_element()) is not None:
-                yield element
-            if transition.episode_end:  # truncation (:199-200)
-                self._trajectory.clear()
+        for window in self._windows(transition):
+            yield self._make_replay_element(window)
+
+    # ---- frame store bookkeeping ----------------------------------------------------------------------
+    # Invariant: every frame id a live element or the trajectory refers to lies in [next id - n_frames, next id), so
+    # writing id f into ring slot f % n_frames never overwrites a frame still in use.  An id leaves that set for good
+    # (the trajectory only drops entries, elements are evicted in FIFO order), so its smallest member never decreases.
+    _frame_store_type = _FrameStore  # anything with put_frame / put_element / grow / n_frames (a host model in tests)
+
+    def _open_frame_store(self, frame: np.ndarray) -> _FrameStore:
+        cap, stack = self._max_capacity, self._stack_size
+        n_frames = cap + cap // 64 + stack + self._update_horizon
+        return self._frame_store_type(cap, frame.shape, frame.dtype, stack, n_frames, self._device)
+
+    def _lowest_frame_in_use(self) -> int:
+        ids = [f for f in self._frame_ids if f is not None]
+        if self._live_min:
+            ids.append(self._live_min[0][1])
+        return min(ids, default=self._next_frame_id)
+
+    def _new_frame_id(self, observation) -> int:
+        store, f = self._store, self._next_frame_id
+        lo = self._lowest_frame_in_use()
+        if f - lo >= store.n_frames:  # many short episodes: more frames in use than the ring holds
+            n_frames = store.n_frames
+            while f - lo >= n_frames:
+                n_frames = (5 * n_frames + 3) // 4  # ceil(1.25 n)
+            store.grow(n_frames, lo, f)
+        store.put_frame(f, observation)
+        self._next_frame_id = f + 1
+        return f
+
+    def _add_frames(self, key: int, window) -> None:
+        pivot, positions = window
+        while self._live_min and self._live_min[0][0] <= key - self._max_capacity:  # the element `key` replaces
+            self._live_min.popleft()
+        for t in sorted({t for t in positions if t >= 0}):  # ids in trajectory order, on first use
+            if self._frame_ids[t] is None:
+                self._frame_ids[t] = self._new_frame_id(self._trajectory[t].observation)
+        ids = [self._frame_ids[t] if t >= 0 else -1 for t in positions]
+        action, ret, terminal = self._scalars(pivot)
+        self._store.put_element(key % self._max_capacity, ids, action, ret, terminal, terminal)
+        smallest = min(f for f in ids if f >= 0)
+        while self._live_min and self._live_min[-1][1] >= smallest:
+            self._live_min.pop()
+        self._live_min.append((key, smallest))
 
     # ---- add / sample / update (replay_buffer.py:202-237) -----------------------------------------------
     def add(self, transition: TransitionElement, **kwargs: Any) -> None:
-        for element in self.accumulate(transition):
-            if self._store is None:
-                self._store = _DeviceStore(self._max_capacity, np.shape(element.state),
-                                           np.asarray(element.state).dtype, self._device)
+        for window in self._windows(transition):
             key = ReplayItemID(self.add_count)
-            self._store.put(key % self._max_capacity, element)
+            if self._frame_store:
+                if self._store is None:
+                    self._store = self._open_frame_store(np.asarray(transition.observation))
+                self._add_frames(key, window)
+            else:
+                element = self._make_replay_element(window)
+                if self._store is None:
+                    self._store = _DeviceStore(self._max_capacity, np.shape(element.state),
+                                               np.asarray(element.state).dtype, self._device)
+                self._store.put(key % self._max_capacity, element)
             self._sampling_distribution.add(key, **kwargs)
             self.add_count += 1
             if self.add_count > self._max_capacity:

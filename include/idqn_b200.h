@@ -240,6 +240,27 @@ int idqn_replay_gather_host(idqn_replay* r, const int64_t* slots_host, int n, vo
 int idqn_learn_from_replay(idqn_handle* h, idqn_replay* r, const int64_t* slots_host, int n, int state_is_u8,
                            float* losses_host);
 
+/* ------------------------------------------------------------------------------------------------
+ * Frame store: ReplayBuffer(compress=True) in spirit (replay_buffer.py:36-57,204-205) -- each observation once in HBM.
+ * A ring of n_frames frames of frame_bytes each (frame id f at ring slot f % n_frames) and, per element slot, 2*stack
+ * frame ids: the state's stack positions, then next_state's (-1 = a zero frame, replay_buffer.py:125,136).  Value
+ * v * stack + p of a stack (value_bytes bytes each) is value v of the frame at position p (the stack is the last axis,
+ * :168-171).  The same handle type as the element store; idqn_replay_destroy,
+ * idqn_replay_gather_host and idqn_learn_from_replay take both (their element size is frame_bytes * stack), while
+ * idqn_replay_put refuses a frame store with IDQN_EINVAL.  A write into a ring slot or element row that a step
+ * enqueued by idqn_learn_from_replay (losses_host == NULL) may still read waits for that step. */
+int idqn_replay_create_frames(int64_t n_slots, int64_t frame_bytes, int stack, int value_bytes, int64_t n_frames,
+                              int device, idqn_replay** out);
+/* ReplayBuffer.add (:207-210), the observation half: frame `frame_id` into ring slot frame_id % n_frames */
+int idqn_replay_put_frame(idqn_replay* r, int64_t frame_id, const void* frame_host);
+/* ReplayBuffer.add (:207-210), the element half: the frame ids and scalars of one element into `slot` */
+int idqn_replay_put_element(idqn_replay* r, int64_t slot, const int64_t* frame_ids_host, int32_t action, double reward,
+                            uint8_t is_terminal, uint8_t episode_end);
+/* no reference counterpart (its store is a dict, replay_buffer.py:89): a ring of n_frames > the current count; the frames
+ * of ids [live_lo, live_hi) (at most the current count) move to their new slots, the old ring is freed once every step
+ * reading it has completed */
+int idqn_replay_grow_frames(idqn_replay* r, int64_t n_frames, int64_t live_lo, int64_t live_hi);
+
 #ifdef __cplusplus
 }
 #endif
