@@ -56,6 +56,7 @@ SYMBOLS = {
     "idqn_set_loss_accumulation": (_I, [_P, _I]),
     "idqn_read_cumulated_losses": (_I, [_P, _P, _I]),
     "idqn_read_td_abs": (_I, [_P, _P]),
+    "idqn_write_cumulated_losses": (_I, [_P, _P]),
     "idqn_kernels_per_step": (_I, [_P]),
     "idqn_profile_step": (_I, [_P, _I, _I, _P, _P, C.POINTER(_I)]),
     "idqn_debug_timeline": (_I, [_P, _I]),
@@ -90,6 +91,7 @@ SYMBOLS = {
     "idqn_sumtree_set_at_max": (_I, [_P, C.c_int32]),
     "idqn_sumtree_update_from_learner": (_I, [_P, _P, _P, _I]),
     "idqn_sumtree_nodes_ptr": (_P, [_P]),
+    "idqn_sumtree_write_nodes": (_I, [_P, _P, C.c_double]),
     "idqn_replay_create": (_I, [_I64, _I64, _I, C.POINTER(_P)]),
     "idqn_replay_destroy": (_I, [_P]),
     "idqn_replay_put": (_I, [_P, _I64, _P, _P, C.c_int32, C.c_double, C.c_uint8, C.c_uint8]),
@@ -99,6 +101,12 @@ SYMBOLS = {
     "idqn_replay_put_frame": (_I, [_P, _I64, _P]),
     "idqn_replay_put_element": (_I, [_P, _I64, _P, C.c_int32, C.c_double, C.c_uint8, C.c_uint8]),
     "idqn_replay_grow_frames": (_I, [_P, _I64, _I64, _I64]),
+    "idqn_replay_read_frames": (_I, [_P, _I64, _I64, _P]),
+    "idqn_replay_write_frames": (_I, [_P, _I64, _I64, _P]),
+    "idqn_replay_read_slots": (_I, [_P, _I64, _I64, _P, _P, _P, _P, _P, _P]),
+    "idqn_replay_write_slots": (_I, [_P, _I64, _I64, _P, _P, _P, _P, _P, _P]),
+    "idqn_replay_digest": (_I, [_P, _I64, _I64, _I64, _P]),
+    "idqn_replay_stream": (_P, [_P]),
 }
 
 _lock = threading.Lock()

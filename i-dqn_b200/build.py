@@ -10,7 +10,7 @@ from concurrent.futures import ThreadPoolExecutor
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libidqn_b200.so")
-SOURCES = ["net.cu", "sumtree.cu", "replay.cu", "peer.cu"]
+SOURCES = ["net.cu", "sumtree.cu", "replay.cu", "peer.cu", "checkpoint.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v",

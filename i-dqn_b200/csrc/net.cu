@@ -1813,6 +1813,13 @@ extern "C" int idqn_read_cumulated_losses(idqn_handle* h, double* sums, int rese
   CK(cudaStreamSynchronize(h->stream));
   return IDQN_OK;
 }
+extern "C" int idqn_write_cumulated_losses(idqn_handle* h, const double* sums) {
+  REQUIRE(h && sums, "null argument");
+  CK(cudaSetDevice(h->cfg.device));
+  CK(cudaMemcpyAsync(h->loss_sum, sums, sizeof(double) * h->K, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return IDQN_OK;
+}
 
 // the target events move the bf16 planes together with their fp32 masters
 // The three target events move the bf16 planes together with the fp32 arenas: planes that are still stale (arena

@@ -336,6 +336,17 @@ extern "C" int idqn_sumtree_read_nodes(idqn_sumtree* t, double* nodes) {
   return IDQN_OK;
 }
 
+// restore of a saved tree: the nodes are uploaded as they were read, not rebuilt through `set` (a node's f64 value
+// depends on the order of the adds that made it)
+extern "C" int idqn_sumtree_write_nodes(idqn_sumtree* t, const double* nodes, double max_recorded) {
+  REQUIRE(t && nodes, "bad argument");
+  CK(cudaSetDevice(t->device));
+  CK(cudaMemcpyAsync(t->nodes, nodes, sizeof(double) * t->n_nodes, cudaMemcpyHostToDevice, t->stream));
+  CK(cudaMemcpyAsync(t->d_maxrec, &max_recorded, sizeof(double), cudaMemcpyHostToDevice, t->stream));
+  CK(cudaStreamSynchronize(t->stream));
+  return IDQN_OK;
+}
+
 template <bool SCALE>
 static int query_impl(idqn_sumtree* t, const double* targets, int32_t* out, int64_t n) {
   REQUIRE(t && targets && out && n >= 0, "bad argument");

@@ -13,13 +13,20 @@ Same signature, same control flow, same bookkeeping as the reference.  What diff
   acting steps hide behind one learning step.
 
 ``p`` needs: n_epochs, n_training_steps_per_epoch, n_initial_samples, epsilon_end, epsilon_duration, horizon; optional
-``wandb`` (anything with ``.log(dict)``) and ``save`` (callable(p, returns, lengths, model), the reference's save_data).
+``wandb`` (anything with ``.log(dict)``), ``save`` (callable(p, returns, lengths, model), the reference's save_data) and
+``checkpoint_dir``: after every epoch ``<checkpoint_dir>/<epoch>/`` receives the agent, the replay buffer (with its
+sampler) and the loop state, and ``train`` resumes from the newest complete checkpoint there.  Only the newest
+``rb._checkpoint_duration`` checkpoints are kept.  An epoch ends right after an episode ended, so the environment has
+just been reset and nothing of it is saved: ``env`` stays the caller's object (its own random state is not restored).
 """
 from __future__ import annotations
+
+import os
 
 import numpy as np
 
 from .. import _prng
+from .. import checkpoint as ckpt
 from ..sample_collection.utils import collect_single_sample
 
 
@@ -43,8 +50,21 @@ def train(key, p: dict, agent, env, rb):
     env.reset()
     episode_returns_per_epoch = [[0]]
     episode_lengths_per_epoch = [[0]]
+    first_epoch = 0
+    root = p.get("checkpoint_dir")
+    if root is not None and (latest := ckpt.latest_checkpoint(root)) is not None:
+        ckpt.verify(latest)
+        agent.load(os.path.join(latest, "agent"))
+        rb.load(os.path.join(latest, "replay"))
+        loop = ckpt.read_json(os.path.join(latest, "loop.json"))
+        first_epoch, n_training_steps = loop["next_epoch"], loop["n_training_steps"]
+        key = np.asarray(loop["key"], np.uint32)
+        episode_returns_per_epoch, episode_lengths_per_epoch = loop["returns"], loop["lengths"]
+        if len(episode_returns_per_epoch) == first_epoch:  # saved after what was then the last epoch
+            episode_returns_per_epoch.append([0])
+            episode_lengths_per_epoch.append([0])
 
-    for idx_epoch in range(p["n_epochs"]):
+    for idx_epoch in range(first_epoch, p["n_epochs"]):
         n_training_steps_epoch = 0
         has_reset = False
 
@@ -76,6 +96,15 @@ def train(key, p: dict, agent, env, rb):
             episode_lengths_per_epoch.append([0])
         if p.get("save") is not None:
             p["save"](p, episode_returns_per_epoch, episode_lengths_per_epoch, agent.get_model())
+        if root is not None:
+            tmp = ckpt.begin(root, str(idx_epoch))
+            agent.save(os.path.join(tmp, "agent"))  # waits for the learner steps still in flight
+            rb.save(os.path.join(tmp, "replay"))
+            ckpt.write_json(os.path.join(tmp, "loop.json"), {
+                "next_epoch": idx_epoch + 1, "n_training_steps": n_training_steps,
+                "key": [int(k) for k in _prng.as_key(key)],
+                "returns": episode_returns_per_epoch, "lengths": episode_lengths_per_epoch})
+            ckpt.commit(root, str(idx_epoch), keep=rb._checkpoint_duration)
     return episode_returns_per_epoch, episode_lengths_per_epoch
 
 

@@ -8,12 +8,14 @@ agent's methods moves no data.  Host pytrees (nested dicts of numpy arrays, flax
 accepted everywhere the reference accepts a pytree and make the call pure-functional, as in the reference."""
 from __future__ import annotations
 
+import os
 from typing import Any, Dict, Optional, Tuple
 
 import numpy as np
 
 from .. import _lib as L
 from .. import _prng
+from .. import checkpoint as ckpt
 from ._engine import EmptyState, Engine, ScaleByAdamState, Tree, CountView, _get
 from .architectures.dqn import DQNNet
 
@@ -258,6 +260,54 @@ class iDQN:
     def get_model(self):
         """idqn.py:133-134 — host numpy copy in the flax layout, so the pickles stay interchangeable."""
         return {"params": self._engine.download_tree(L.ONLINE, squeezed=self._squeeze)}
+
+    # ---- checkpoint (no reference counterpart: the reference only pickles get_model()) --------------------------------
+    _TREES = (("online", L.ONLINE), ("target", L.TARGET), ("mu", L.MU), ("nu", L.NU))
+
+    def _checkpoint_meta(self) -> dict:
+        """What a checkpoint must agree on: the model constructor fields and the schedule (not device / flags)."""
+        c = self._ctor
+        return {"class": type(self).__name__, "observation_dim": [int(d) for d in np.atleast_1d(c["observation_dim"])],
+                "n_actions": int(c["n_actions"]), "n_networks": self.n_networks,
+                "features": [int(f) for f in c["features"]], "architecture_type": c["architecture_type"],
+                "learning_rate": float(c["learning_rate"]), "gamma": float(c["gamma"]),
+                "update_horizon": int(c["update_horizon"]), "adam_eps": float(c["adam_eps"]),
+                "batch_size": int(c["batch_size"]), "update_to_data": int(self.update_to_data),
+                "target_update_frequency": int(self.target_update_frequency),
+                "target_sync_frequency": int(getattr(self, "target_sync_frequency", self.target_update_frequency))}
+
+    def save(self, directory: str) -> None:
+        """Online and target parameters and the Adam moments in the flax layout (one .npz each, leaves named
+        "Module.kind"), Adam's count and the device loss sums.  Waits for learner steps still in flight."""
+        os.makedirs(directory, exist_ok=True)
+        e = self._engine
+        for name, which in self._TREES:
+            leaves = {}
+            for i, info in enumerate(e.leaves):
+                a = e.download_leaf(which, i)
+                leaves[info["module"].replace("/", ".") + "." + info["kind"]] = a[0] if self._squeeze else a
+            np.savez(os.path.join(directory, name + ".npz"), **leaves)
+        np.save(os.path.join(directory, "count.npy"), e.get_count())
+        np.save(os.path.join(directory, "cumulated_losses.npy"), e.cumulated_losses(reset=False))
+        ckpt.write_json(os.path.join(directory, "agent.json"), self._checkpoint_meta())
+
+    def load(self, directory: str) -> None:
+        """Restore what ``save`` wrote; ValueError naming the first field in which the checkpoint's agent differs."""
+        saved = ckpt.read_json(os.path.join(directory, "agent.json"))
+        for k, v in self._checkpoint_meta().items():
+            if saved.get(k) != v:
+                raise ValueError(f"agent checkpoint has {k}={saved.get(k)!r}, this agent {v!r}")
+        e = self._engine
+        for name, which in self._TREES:
+            with np.load(os.path.join(directory, name + ".npz")) as z:
+                for i, info in enumerate(e.leaves):
+                    a = z[info["module"].replace("/", ".") + "." + info["kind"]]
+                    e.upload_leaf(which, i, a[None] if self._squeeze else a)  # the bf16 planes are rebuilt from these
+        e.set_count(np.load(os.path.join(directory, "count.npy")))
+        sums = np.ascontiguousarray(np.load(os.path.join(directory, "cumulated_losses.npy")), np.float64)
+        if sums.shape != (e.K,):
+            raise ValueError(f"agent checkpoint has {sums.shape[0]} loss sums, this agent {e.K} heads")
+        L.check(e.lib.idqn_write_cumulated_losses(e.h, L.ptr(sums)))
 
 
 def _host(tree):

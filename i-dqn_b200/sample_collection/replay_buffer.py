@@ -19,6 +19,7 @@ from __future__ import annotations
 import collections
 import ctypes as C
 import dataclasses
+import os
 import typing
 import weakref
 import zlib
@@ -27,6 +28,7 @@ from typing import Any, Iterable, Iterator, Optional
 import numpy as np
 
 from .. import _lib as L
+from .. import checkpoint as ckpt
 from . import ReplayItemID
 
 
@@ -70,7 +72,52 @@ class ReplayElement:  # replay_buffer.py:26-69
         return self.replace(state=self.uncompress(self.state), next_state=self.uncompress(self.next_state))
 
 
-class _DeviceStore:
+class _Store:
+    """What both device stores share: the host gather, and the bulk slot transfers and digest of a checkpoint."""
+
+    def gather(self, slots: np.ndarray):
+        n = len(slots)
+        slots = np.ascontiguousarray(slots, dtype=np.int64)
+        s = np.empty((n,) + self.shape, self.dtype)
+        s2 = np.empty((n,) + self.shape, self.dtype)
+        a, r = np.empty(n, np.int32), np.empty(n, np.float64)
+        d, e = np.empty(n, np.uint8), np.empty(n, np.uint8)
+        L.check(self.lib.idqn_replay_gather_host(self.h, L.ptr(slots), n, L.ptr(s), L.ptr(s2), L.ptr(a), L.ptr(r),
+                                                 L.ptr(d), L.ptr(e)))
+        return s, s2, a.astype(np.int64), r, d.astype(bool), e.astype(bool)
+
+    def _slot_stacks(self, n: int):
+        raise NotImplementedError
+
+    def read_slots(self, lo: int, n: int):
+        """(state stacks or frame-id rows, next_state stacks or None, action i32, reward f64, terminal u8,
+        episode_end u8) of slots [lo, lo + n)."""
+        s, s2 = self._slot_stacks(n)
+        a, r = np.empty(n, np.int32), np.empty(n, np.float64)
+        d, e = np.empty(n, np.uint8), np.empty(n, np.uint8)
+        L.check(self.lib.idqn_replay_read_slots(self.h, int(lo), int(n), L.ptr(s), None if s2 is None else L.ptr(s2),
+                                                L.ptr(a), L.ptr(r), L.ptr(d), L.ptr(e)))
+        return s, s2, a, r, d, e
+
+    def write_slots(self, lo: int, s, s2, a, r, d, e) -> None:
+        like, like2 = self._slot_stacks(0)
+        s = np.ascontiguousarray(s, like.dtype)
+        s2 = None if like2 is None else np.ascontiguousarray(s2, like2.dtype)
+        a, r = np.ascontiguousarray(a, np.int32), np.ascontiguousarray(r, np.float64)
+        d, e = np.ascontiguousarray(d, np.uint8), np.ascontiguousarray(e, np.uint8)
+        if s.shape[1:] != like.shape[1:] or any(len(x) != len(s) for x in (a, r, d, e)):
+            raise ValueError("slot arrays do not match the store")
+        L.check(self.lib.idqn_replay_write_slots(self.h, int(lo), len(s), L.ptr(s), None if s2 is None else L.ptr(s2),
+                                                 L.ptr(a), L.ptr(r), L.ptr(d), L.ptr(e)))
+
+    def digest(self, n_live: int, id_lo: int = 0, id_hi: int = 0) -> list:
+        """idqn_replay_digest: six digests computed on the device (see include/idqn_b200.h)."""
+        out = np.zeros(6, np.uint64)
+        L.check(self.lib.idqn_replay_digest(self.h, int(n_live), int(id_lo), int(id_hi), L.ptr(out)))
+        return [int(x) for x in out]
+
+
+class _DeviceStore(_Store):
     """Fixed-slot element store in HBM."""
 
     def __init__(self, n_slots: int, obs_shape, obs_dtype, device: int):
@@ -91,19 +138,11 @@ class _DeviceStore:
         L.check(self.lib.idqn_replay_put(self.h, int(slot), L.ptr(s), L.ptr(s2), int(el.action), float(el.reward),
                                          int(bool(el.is_terminal)), int(bool(el.episode_end))))
 
-    def gather(self, slots: np.ndarray):
-        n = len(slots)
-        slots = np.ascontiguousarray(slots, dtype=np.int64)
-        s = np.empty((n,) + self.shape, self.dtype)
-        s2 = np.empty((n,) + self.shape, self.dtype)
-        a, r = np.empty(n, np.int32), np.empty(n, np.float64)
-        d, e = np.empty(n, np.uint8), np.empty(n, np.uint8)
-        L.check(self.lib.idqn_replay_gather_host(self.h, L.ptr(slots), n, L.ptr(s), L.ptr(s2), L.ptr(a), L.ptr(r),
-                                                 L.ptr(d), L.ptr(e)))
-        return s, s2, a.astype(np.int64), r, d.astype(bool), e.astype(bool)
+    def _slot_stacks(self, n: int):
+        return np.empty((n,) + self.shape, self.dtype), np.empty((n,) + self.shape, self.dtype)
 
 
-class _FrameStore:
+class _FrameStore(_Store):
     """Frame store in HBM (idqn_replay_create_frames): a ring of ``n_frames`` observations (frame id ``f`` in ring slot
     ``f % n_frames``) and, per element slot, ``2 * stack`` frame ids (-1: a zero frame)."""
 
@@ -138,7 +177,20 @@ class _FrameStore:
         L.check(self.lib.idqn_replay_grow_frames(self.h, int(n_frames), int(live_lo), int(live_hi)))
         self._n_frames = int(n_frames)
 
-    gather = _DeviceStore.gather
+    def _slot_stacks(self, n: int):
+        return np.empty((n, 2 * self.stack), np.int64), None
+
+    def read_frames(self, id_lo: int, id_hi: int) -> np.ndarray:
+        """frames of ids [id_lo, id_hi) in id order"""
+        out = np.empty((id_hi - id_lo,) + self.frame_shape, self.dtype)
+        L.check(self.lib.idqn_replay_read_frames(self.h, int(id_lo), int(id_hi), L.ptr(out)))
+        return out
+
+    def write_frames(self, id_lo: int, frames) -> None:
+        f = np.ascontiguousarray(frames, dtype=self.dtype)
+        if f.shape[1:] != self.frame_shape:
+            raise ValueError(f"frame shape {f.shape[1:]} differs from the store's {self.frame_shape}")
+        L.check(self.lib.idqn_replay_write_frames(self.h, int(id_lo), int(id_lo) + len(f), L.ptr(f)))
 
 
 class _MemoryView(collections.abc.Mapping):
@@ -374,3 +426,121 @@ class ReplayBuffer:
         if upd is None:
             raise TypeError("update_from_learner needs a PrioritizedSamplingDistribution")
         upd(self.last_keys, engine)
+
+    # ---- checkpoint -----------------------------------------------------------------------------------------------
+    # Dopamine's save/load (the origin of ``checkpoint_duration``, replay_buffer.py:82,93 of the reference, which never
+    # uses it) for the device store: the accumulator, the frame bookkeeping, the live part of the store streamed in
+    # chunks, the sampler and the device-computed digests the load checks what landed in HBM against.
+    _DIGESTS = ("state/frames", "next_state/rows", "action", "reward", "terminal", "episode_end")
+
+    def _config(self) -> dict:
+        return {"max_capacity": int(self._max_capacity), "stack_size": int(self._stack_size),
+                "update_horizon": int(self._update_horizon), "gamma": float(self._gamma),
+                "batch_size": int(self._batch_size), "frame_store": bool(self._frame_store),
+                "sampler": type(self._sampling_distribution).__name__}
+
+    def _slot_files(self):
+        return ("rows" if self._frame_store else "state", "next_state", "action", "reward", "terminal", "episode_end")
+
+    def save(self, directory: str) -> None:
+        """Write this buffer into ``directory`` (created if missing).  Waits for learner steps still reading the store."""
+        os.makedirs(directory, exist_ok=True)
+        join = lambda name: os.path.join(directory, name)
+        traj = list(self._trajectory)
+        meta = {"config": self._config(), "add_count": int(self.add_count), "trajectory": len(traj), "store": None}
+        if traj:
+            np.save(join("trajectory_observation.npy"), np.stack([np.asarray(t.observation) for t in traj]))
+            np.save(join("trajectory_action.npy"), np.asarray([int(t.action) for t in traj], np.int64))
+            np.save(join("trajectory_reward.npy"), np.asarray([float(t.reward) for t in traj], np.float64))
+            np.save(join("trajectory_flags.npy"),
+                    np.asarray([(bool(t.is_terminal), bool(t.episode_end)) for t in traj], np.uint8).reshape(-1, 2))
+        if self._frame_store:
+            meta["frame_ids"] = [-1 if f is None else int(f) for f in self._frame_ids]
+            meta["next_frame_id"] = int(self._next_frame_id)
+            meta["live_min"] = [[int(k), int(f)] for k, f in self._live_min]
+        st = self._store
+        if st is not None:
+            n_live = min(self.add_count, self._max_capacity)
+            lo, hi = (self._lowest_frame_in_use(), self._next_frame_id) if self._frame_store else (0, 0)
+            meta["store"] = {"shape": list(st.frame_shape if self._frame_store else st.shape), "dtype": st.dtype.str,
+                             "n_frames": int(st.n_frames) if self._frame_store else None, "n_live": n_live,
+                             "frames": [lo, hi], "digest": st.digest(n_live, lo, hi)}
+            if self._frame_store:
+                per = ckpt.rows_per_chunk(st.frame_bytes)
+                w = ckpt.NpyWriter(join("frames.npy"), (hi - lo,) + st.frame_shape, st.dtype)
+                for f in range(lo, hi, per):
+                    w.write(st.read_frames(f, min(f + per, hi)))
+                w.close()
+            writers = []
+            per = ckpt.rows_per_chunk(16 * self._stack_size + 14 if self._frame_store else 2 * st.state_bytes + 14)
+            for k in range(0, n_live, per):
+                arrays = st.read_slots(k, min(per, n_live - k))
+                if not writers:
+                    writers = [None if a is None else ckpt.NpyWriter(join(name + ".npy"), (n_live,) + a.shape[1:], a.dtype)
+                               for name, a in zip(self._slot_files(), arrays)]
+                for wr, a in zip(writers, arrays):
+                    if wr is not None:
+                        wr.write(a)
+            for wr in writers:
+                if wr is not None:
+                    wr.close()
+        if getattr(self, "last_keys", None) is not None:
+            np.save(join("last_keys.npy"), np.asarray(self.last_keys))
+        if hasattr(self._sampling_distribution, "save"):
+            self._sampling_distribution.save(join("sampler"))
+        ckpt.write_json(join("replay.json"), meta)
+
+    def load(self, directory: str) -> None:
+        """Restore a buffer written by ``save`` into this one, which must have been just constructed with the same
+        configuration (ValueError otherwise).  The store is re-created at its saved size and its contents are checked
+        against the saved digests on the device (ValueError on a mismatch; the buffer is then unusable)."""
+        join = lambda name: os.path.join(directory, name)
+        meta = ckpt.read_json(join("replay.json"))
+        if self.add_count != 0 or self._store is not None or self._trajectory:
+            raise ValueError("ReplayBuffer.load needs a buffer nothing has been added to")
+        for k, v in self._config().items():
+            if meta["config"][k] != v:
+                raise ValueError(f"replay checkpoint has {k}={meta['config'][k]!r}, this buffer {v!r}")
+        if meta["trajectory"]:
+            obs = np.load(join("trajectory_observation.npy"))
+            act, rew = np.load(join("trajectory_action.npy")), np.load(join("trajectory_reward.npy"))
+            flags = np.load(join("trajectory_flags.npy"))
+            for t in range(meta["trajectory"]):
+                self._trajectory.append(TransitionElement(obs[t], int(act[t]), float(rew[t]), bool(flags[t, 0]),
+                                                          bool(flags[t, 1])))
+        if self._frame_store:
+            self._frame_ids.extend(None if f < 0 else f for f in meta["frame_ids"])
+            self._next_frame_id = meta["next_frame_id"]
+            self._live_min.extend((k, f) for k, f in meta["live_min"])
+        sm = meta["store"]
+        if sm is not None:
+            shape, dtype, n_live = tuple(sm["shape"]), np.dtype(sm["dtype"]), sm["n_live"]
+            lo, hi = sm["frames"]
+            if self._frame_store:
+                st = self._store = self._frame_store_type(self._max_capacity, shape, dtype, self._stack_size,
+                                                          sm["n_frames"], self._device)
+                rd = ckpt.NpyReader(join("frames.npy"))
+                per = ckpt.rows_per_chunk(st.frame_bytes)
+                for f in range(lo, hi, per):
+                    st.write_frames(f, rd.read(min(per, hi - f)))
+                rd.close()
+            else:
+                st = self._store = _DeviceStore(self._max_capacity, shape, dtype, self._device)
+            readers = [ckpt.NpyReader(join(n + ".npy")) if n != "next_state" or not self._frame_store else None
+                       for n in self._slot_files()]
+            per = ckpt.rows_per_chunk(16 * self._stack_size + 14 if self._frame_store else 2 * st.state_bytes + 14)
+            for k in range(0, n_live, per):
+                m = min(per, n_live - k)
+                st.write_slots(k, *[None if rd is None else rd.read(m) for rd in readers])
+            for rd in readers:
+                if rd is not None:
+                    rd.close()
+            got = st.digest(n_live, lo, hi)
+            bad = [n for n, a, b in zip(self._DIGESTS, got, sm["digest"]) if a != b]
+            if bad:
+                raise ValueError(f"replay digest mismatch in {', '.join(bad)}: {directory} does not hold the saved store")
+        self.add_count = meta["add_count"]
+        if os.path.exists(join("last_keys.npy")):
+            self.last_keys = np.load(join("last_keys.npy"))
+        if hasattr(self._sampling_distribution, "load"):
+            self._sampling_distribution.load(join("sampler"))

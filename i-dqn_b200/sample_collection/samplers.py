@@ -5,8 +5,11 @@ recommends (32 numbers per step; numpy *is* the reference's generator, so the st
 SumTree arithmetic of the prioritised sampler runs on the GPU."""
 from __future__ import annotations
 
+import os
+
 import numpy as np
 
+from .. import checkpoint as ckpt
 from . import ReplayItemID
 from .sum_tree import SumTree
 
@@ -36,6 +39,25 @@ class UniformSamplingDistribution:
         picks = self._rng_key.integers(len(self._index_to_key), size=size)
         table = self._index_to_key
         return np.fromiter((table[i] for i in picks), dtype=np.int32, count=size)
+
+    # ---- checkpoint: the key table and the generator state (a reloaded sampler draws the same keys) ----------------
+    def _meta(self) -> dict:
+        return {"type": type(self).__name__}
+
+    def save(self, directory: str) -> None:
+        os.makedirs(directory, exist_ok=True)
+        np.save(os.path.join(directory, "index_to_key.npy"), np.asarray(self._index_to_key, np.int64))
+        ckpt.write_json(os.path.join(directory, "sampler.json"),
+                        {**self._meta(), "bit_generator": self._rng_key.bit_generator.state})
+
+    def load(self, directory: str) -> None:
+        meta = ckpt.read_json(os.path.join(directory, "sampler.json"))
+        for k, v in self._meta().items():
+            if meta.get(k) != v:
+                raise ValueError(f"sampler checkpoint has {k}={meta.get(k)!r}, this sampler {v!r}")
+        self._index_to_key = [int(k) for k in np.load(os.path.join(directory, "index_to_key.npy"))]
+        self._key_to_index = {k: i for i, k in enumerate(self._index_to_key)}
+        self._rng_key.bit_generator.state = meta["bit_generator"]
 
 
 class PrioritizedSamplingDistribution(UniformSamplingDistribution):
@@ -91,6 +113,22 @@ class PrioritizedSamplingDistribution(UniformSamplingDistribution):
             self._sum_tree.set(np.asarray([hole, tail], dtype=np.int32),
                                np.asarray([self._sum_tree.get(tail), 0.0], dtype=np.float64))
         super().remove(key)
+
+    def _meta(self) -> dict:
+        return {**super()._meta(), "max_capacity": int(self._max_capacity),
+                "priority_exponent": float(self._priority_exponent)}
+
+    def save(self, directory: str) -> None:
+        super().save(directory)
+        np.save(os.path.join(directory, "sum_tree_nodes.npy"), self._sum_tree._nodes)
+        ckpt.write_json(os.path.join(directory, "sum_tree.json"),
+                        {"max_recorded_priority": self._sum_tree.max_recorded_priority})
+
+    def load(self, directory: str) -> None:
+        """The tree's nodes are uploaded as saved (``write_nodes``), never rebuilt through ``set``."""
+        super().load(directory)
+        self._sum_tree.write_nodes(np.load(os.path.join(directory, "sum_tree_nodes.npy")),
+                                   ckpt.read_json(os.path.join(directory, "sum_tree.json"))["max_recorded_priority"])
 
     def sample(self, size: int):
         # samplers.py:105-108: an all-zero tree falls back to the uniform sampler (the reference spells the intent as

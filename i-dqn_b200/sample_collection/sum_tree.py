@@ -40,6 +40,14 @@ class SumTree:
         L.check(self._lib.idqn_sumtree_read_nodes(self._h, L.ptr(out)))
         return out
 
+    def write_nodes(self, nodes, max_recorded_priority: float) -> None:
+        """Restore a saved tree: ``_nodes`` and ``max_recorded_priority`` uploaded unchanged.  (Replaying ``set`` on the
+        leaves would not give the same nodes: each f64 node depends on the order of the adds that built it.)"""
+        n = np.ascontiguousarray(nodes, dtype=np.float64)
+        if n.shape != (self._n_nodes,):
+            raise ValueError(f"{n.shape} nodes for a tree of {self._n_nodes}")
+        L.check(self._lib.idqn_sumtree_write_nodes(self._h, L.ptr(n), float(max_recorded_priority)))
+
     def set(self, indices, values) -> None:  # sum_tree.py:20-47
         if isinstance(indices, (int, np.integer)):
             indices = np.asarray([indices], np.int32)

@@ -136,6 +136,8 @@ int idqn_set_loss_accumulation(idqn_handle* h, int on);
 int idqn_read_td_abs(idqn_handle* h, float* out_host);
 /* idqn.py:72,82-87: device-side sum of the per-head losses since the last reset */
 int idqn_read_cumulated_losses(idqn_handle* h, double* sums_host, int reset);
+/* its inverse (restore of a checkpoint): the K sums become sums_host */
+int idqn_write_cumulated_losses(idqn_handle* h, const double* sums_host);
 
 /* measurement aids (no reference counterpart): kernels one step launches, and one un-graphed step with a CUDA
  * event after every launch -> ms[i] / names[32*i..] per kernel, in launch order.  It runs on the batch the LAST host-batch
@@ -222,6 +224,10 @@ int idqn_sumtree_set_at_max(idqn_sumtree* t, int32_t leaf);
  * Only priority_exponent == 1 is served here (the reference's array power has to stay numpy's, bit for bit). */
 int idqn_sumtree_update_from_learner(idqn_sumtree* t, idqn_handle* h, const int32_t* leaves_host, int n);
 void* idqn_sumtree_nodes_ptr(idqn_sumtree* t);
+/* restore of a checkpoint: the whole _nodes array (idqn_sumtree_num_nodes doubles, as idqn_sumtree_read_nodes returned
+ * it) and max_recorded_priority, uploaded unchanged -- a node's f64 value depends on the order of the adds that built it,
+ * so replaying `set` on the leaves would not reproduce it */
+int idqn_sumtree_write_nodes(idqn_sumtree* t, const double* nodes_host, double max_recorded);
 
 /* ------------------------------------------------------------------------------------------------
  * Device-resident replay store (slimdqn/sample_collection/replay_buffer.py:89,202-230): fixed slots of
@@ -260,6 +266,35 @@ int idqn_replay_put_element(idqn_replay* r, int64_t slot, const int64_t* frame_i
  * of ids [live_lo, live_hi) (at most the current count) move to their new slots, the old ring is freed once every step
  * reading it has completed */
 int idqn_replay_grow_frames(idqn_replay* r, int64_t n_frames, int64_t live_lo, int64_t live_hi);
+
+/* ------------------------------------------------------------------------------------------------
+ * Checkpoint of a replay store (no reference counterpart: its checkpoint_duration argument is never used,
+ * replay_buffer.py:82,93).  Each transfer first waits for the store's stream and for every learner step that may
+ * still read the store, then copies in chunks through a pinned staging buffer of the store; host buffers may be
+ * pageable.  A restore re-creates the store at its saved size (idqn_replay_create_frames takes n_frames). */
+/* frame ids [id_lo, id_hi) in id order (frame id f at ring slot f % n_frames; a range that wraps is two copies);
+ * id_hi - id_lo <= n_frames, otherwise IDQN_EINVAL */
+int idqn_replay_read_frames(idqn_replay* r, int64_t id_lo, int64_t id_hi, void* dst_host);
+int idqn_replay_write_frames(idqn_replay* r, int64_t id_lo, int64_t id_hi, const void* src_host);
+/* slots [slot_lo, slot_lo + n): element store: state_or_rows / next_state are the two stacks ([n][state_bytes]);
+ * frame store: state_or_rows is the int64 [n][2*stack] frame-id rows and next_state must be NULL (write_slots also
+ * sets the host mirror of the rows) */
+int idqn_replay_read_slots(idqn_replay* r, int64_t slot_lo, int64_t n, void* state_or_rows_host,
+                           void* next_state_host, int32_t* action_host, double* reward_host, uint8_t* is_terminal_host,
+                           uint8_t* episode_end_host);
+int idqn_replay_write_slots(idqn_replay* r, int64_t slot_lo, int64_t n, const void* state_or_rows_host,
+                            const void* next_state_host, const int32_t* action_host, const double* reward_host,
+                            const uint8_t* is_terminal_host, const uint8_t* episode_end_host);
+/* one 64-bit digest per logical array of the store, computed on the device:
+ *   out[0]: element store: state stacks of slots [0, n_live_slots); frame store: frames [id_lo, id_hi) in id order,
+ *           each zero-padded to a multiple of 8 bytes (id_lo / id_hi are ignored by an element store)
+ *   out[1]: next_state stacks / frame-id rows of the same slots;  out[2..5]: action, reward, terminal, episode_end
+ * For a byte stream of length L zero-padded to N little-endian 64-bit words w_i:
+ *   digest = (sum_i splitmix64(w_i + (i + 1) * 0x9E3779B97F4A7C15)) mod 2^64  XOR  splitmix64(L)
+ * It depends neither on the grid nor on the ring's size. */
+int idqn_replay_digest(idqn_replay* r, int64_t n_live_slots, int64_t id_lo, int64_t id_hi, uint64_t out[6]);
+/* the store's CUDA stream (cudaStream_t): its transfers and the digest run on it (events around the digest) */
+void* idqn_replay_stream(idqn_replay* r);
 
 #ifdef __cplusplus
 }
