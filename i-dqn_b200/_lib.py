@@ -76,7 +76,8 @@ SYMBOLS = {
     "idqn_apply_host": (_I, [_P, _I, _I, _P, _I, _I, _P]),
     "idqn_best_action": (_I, [_P, _I, _I, _P, _I, C.POINTER(C.c_int32)]),
     "idqn_select_action": (_I, [_P, _P, _I, C.c_uint32, C.c_uint32, _I, C.c_float, C.POINTER(C.c_int32), _P]),
-    "idqn_prng": (_I, [_I, C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, _P]),
+    "idqn_select_actions": (_I, [_P, _P, _I, _I, _P, _I, C.c_float, _P, _P]),
+    "idqn_prng":(_I, [_I, C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, _P]),
     "idqn_sumtree_create": (_I, [_I64, _I, C.POINTER(_P)]),
     "idqn_sumtree_destroy": (_I, [_P]),
     "idqn_sumtree_depth": (_I, [_P]),

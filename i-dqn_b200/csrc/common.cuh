@@ -240,6 +240,17 @@ struct idqn_handle {
   int32_t* best_idx;     // device word receiving the argmax of best_action
   cudaGraphExec_t* act_graph;  // [K] best_action fast path of head k as ONE graph launch (H2D state, 7 kernels, D2H action)
   uint8_t* h_state;      // pinned staging of the acting state (source of the graphs' H2D node)
+  // idqn_select_actions, allocated on its first call: per chunk of up to B environments, a pinned staging block (act
+  // codes, then the states) and the actions it gets back; one device copy of a block and the chunk's actions
+  uint8_t* h_vact;       // pinned [chunks][vact_block]
+  int32_t* h_vout;       // pinned [chunks * B]
+  size_t h_vact_bytes;
+  int64_t vact_chunks;   // chunks h_vact / h_vout hold
+  uint8_t* d_vact;       // [vact_block]
+  int32_t* d_vout;       // [B]
+  cudaGraph_t vact_graph[8];          // fast path, one per padded chunk size 2^i (kept: its memcpy nodes are re-pointed)
+  cudaGraphExec_t vact_exec[8];
+  cudaGraphNode_t vact_h2d[8], vact_d2h[8];
   // pinned host scratch
   float* h_loss;
   int32_t* h_i32;

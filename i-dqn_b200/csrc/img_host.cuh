@@ -495,13 +495,14 @@ static cudaError_t img_set_smem(Kern kern, size_t bytes) {
   return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IMG_SMEM_OPTIN);
 }
 
-// single_state: only the first image of `state` (best_action); otherwise the whole batch of state and next_state
-static int img_launch_s2d(idqn_handle* h, int x_u8, bool single_state = false) {
+// act_imgs > 0: only the first act_imgs images of `state` (acting); otherwise the whole batch of state and next_state
+static int img_launch_s2d(idqn_handle* h, int x_u8, int act_imgs = 0) {
   ImgHost* H = (ImgHost*)h->img_host;
   img::S2dArgs a = H->s2d;
   a.u8 = x_u8;
+  const bool single_state = act_imgs > 0;
   a.tl_id = single_state ? -1 : tl_next(h);
-  if (single_state) a.imgs = 1, a.n_src = 1;
+  if (single_state) a.imgs = act_imgs, a.n_src = 1;
   a.src[0] = h->s, a.src[1] = h->s2;  // the staging set of this step (idqn_submit_batch_host points it at its slot)
   a.slots = nullptr, a.ring = nullptr;
   if (h->rsrc_on) {  // idqn_learn_from_replay: frames read from the replay slots in place, scalars gathered here

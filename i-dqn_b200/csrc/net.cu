@@ -476,6 +476,29 @@ __global__ void argmax_kernel(const float* __restrict__ q, int A, int32_t* out) 
   }
 }
 
+// idqn_select_actions: one warp per environment.  code[i] >= 0: greedy, out[i] = the first argmax of the Q row code[i]
+// (argmax_kernel's result, NaN included: a NaN at index 0 wins, any later NaN is never taken); code[i] < 0: exploring,
+// out[i] = -1 - code[i], the random action drawn on the host.  code == nullptr: every environment is greedy on row i.
+__global__ void act_select_kernel(const float* __restrict__ q, int A, const int32_t* __restrict__ code, int n,
+                                  int32_t* __restrict__ out) {
+  const int i = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (i >= n) return;
+  const int c = code ? code[i] : i;
+  if (c < 0) {
+    if (lane == 0) out[i] = -1 - c;
+    return;
+  }
+  const float* row = q + (int64_t)c * A;
+  float v = lane < A ? row[lane] : 0.f;
+  int idx = lane < A && !(lane > 0 && v != v) ? lane : HEAD_MAXA;  // HEAD_MAXA: no candidate
+  for (int o = 16; o; o >>= 1) {
+    const float v2 = __shfl_xor_sync(0xffffffffu, v, o);
+    const int i2 = __shfl_xor_sync(0xffffffffu, idx, o);
+    if (i2 < HEAD_MAXA && (idx == HEAD_MAXA || v2 > v || (v2 == v && i2 < idx) || (i2 == 0 && v2 != v2))) v = v2, idx = i2;
+  }
+  if (lane == 0) out[i] = idx;
+}
+
 // ------------------------------------------------------------------------------------------
 // every kernel launch of the step goes through mark(): counts launches and, when profiling, drops an event
 // timeline slot of the launch about to be enqueued (its index inside the step), -1 when the timeline is off
@@ -1557,6 +1580,14 @@ extern "C" int idqn_destroy(idqn_handle* h) {
     delete[] h->act_graph;
   }
   if (h->h_state) cudaFreeHost(h->h_state);
+  for (int i = 0; i < 8; ++i) {
+    if (h->vact_exec[i]) cudaGraphExecDestroy(h->vact_exec[i]);
+    if (h->vact_graph[i]) cudaGraphDestroy(h->vact_graph[i]);
+  }
+  if (h->h_vact) cudaFreeHost(h->h_vact);
+  if (h->h_vout) cudaFreeHost(h->h_vout);
+  if (h->d_vact) cudaFree(h->d_vact);
+  if (h->d_vout) cudaFree(h->d_vout);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   for (int i = 0; i < 2; ++i)
     if (h->ev_join[i]) cudaEventDestroy(h->ev_join[i]);
@@ -1933,20 +1964,25 @@ static int enqueue_apply(idqn_handle* h, int which, int head, int u8, int n) {
 // best_action fast path (idqn.py:126-131 at Atari shapes): the single uint8 state runs through the SAME image-resident conv
 // kernels, weight-streaming Dense_0 kernel and head kernel as the learning step, as (online head, image 0) of the training
 // layout -- the step's activation buffers are scratch between steps.  q[(head * B + 0) * A ..] receives the Q-values.
+// idqn_select_actions runs the same kernels over images [0, imgs) of the online heads [head0, head0 + heads): every
+// (net, image) unit is computed exactly as it is alone, so q[(head * B + i) * A ..] equals the single-state row.
 static bool apply_fast_ok(const idqn_handle* h, int which, int u8) {
   if (!h->img_on || !h->img_host || which != IDQN_ONLINE || !u8 || h->n_layers != IDQN_IMG_LAYERS + 2) return false;
   const ImgHost* H = (const ImgHost*)h->img_host;
   return H->dense_on && H->dfwd.splits > 1 && !(h->cfg.flags & IDQN_F_SLOW_APPLY);
 }
-static int enqueue_apply_fast(idqn_handle* h, int head) {
+static int enqueue_apply_fast(idqn_handle* h, int head0, int heads = 1, int imgs = 1) {
   ImgHost* H = (ImgHost*)h->img_host;
   const int keep = h->n_launch, prof = h->prof_on;  // launch accounting / profiling belong to the learning step
   h->prof_on = 0;
+  // units (net, image) of conv1/conv2 and (net, sample) pairs of the head: net-major, so the window from (head0, 0) to
+  // (head0 + heads - 1, imgs - 1) also covers images >= imgs of the heads before the last (their results are not read)
+  const int pairs = (heads - 1) * h->B + imgs, dunits = H->dfwd.tiles * H->dfwd.splits;
   int rc = refresh_planes(h);
-  if (!rc) rc = img_launch_s2d(h, 1, true);
-  if (!rc) rc = img_launch_taps(h, 0, false, 1, 0, H->fwd[0].n_hg);  // every online head group of image 0
-  for (int li = 1; li < IDQN_IMG_LAYERS && !rc; ++li) rc = img_launch_taps(h, li, false, 2, head * h->B, 1);
-  if (!rc) rc = dense_launch(h, false, false, head * H->dfwd.tiles * H->dfwd.splits, H->dfwd.tiles * H->dfwd.splits);
+  if (!rc) rc = img_launch_s2d(h, 1, imgs);
+  if (!rc) rc = img_launch_taps(h, 0, false, 1, 0, imgs * H->fwd[0].n_hg);  // every online head group of images [0, imgs)
+  for (int li = 1; li < IDQN_IMG_LAYERS && !rc; ++li) rc = img_launch_taps(h, li, false, 2, head0 * h->B, pairs);
+  if (!rc) rc = dense_launch(h, false, false, head0 * dunits, heads * dunits);
   if (!rc) {
     const int L = h->n_layers;
     const Layer& l = h->layers[L - 1];
@@ -1961,8 +1997,8 @@ static int enqueue_apply_fast(idqn_handle* h, int head) {
     a.part = H->dfwd.part, a.ptiles = H->dfwd.tiles, a.psplits = H->dfwd.splits, a.pb_off = h->layers[L - 2].b_off;
     a.hbias_off = -1;
     a.tl_id = -1;
-    a.cta0 = head * h->B;
-    CK(launch_pdl(h->pdl, head_q_kernel, dim3(1), dim3(128), 0, h->stream, a));
+    a.cta0 = head0 * h->B;
+    CK(launch_pdl(h->pdl, head_q_kernel, dim3(pairs), dim3(128), 0, h->stream, a));
   }
   h->n_launch = keep, h->prof_on = prof;
   return rc;
@@ -2129,6 +2165,173 @@ extern "C" int idqn_select_action(idqn_handle* h, const void* state, int u8, uin
     return IDQN_OK;  // no device work at all on an exploring step
   }
   return idqn_best_action(h, IDQN_ONLINE, head, state, u8, action);
+}
+
+// ---- idqn_select_actions: the acting step of N environments ---------------------------------------------------------
+// Staging block of one chunk (host and device alike): the B act codes of act_select_kernel, then the chunk's states.
+static size_t vact_states_off(const idqn_handle* h) { return ((size_t)h->B * sizeof(int32_t) + 255) / 256 * 256; }
+static size_t vact_block(const idqn_handle* h) {
+  return (vact_states_off(h) + (size_t)h->B * h->in_elems * 4 + 255) / 256 * 256;
+}
+
+// pinned staging for `chunks` chunks (grown, never shrunk; nothing of ours is in flight between calls)
+static int vact_reserve(idqn_handle* h, int64_t chunks) {
+  if (!h->d_vact) {
+    CK(cudaMalloc(&h->d_vact, vact_block(h)));
+    CK(cudaMalloc(&h->d_vout, sizeof(int32_t) * h->B));
+  }
+  if (chunks <= h->vact_chunks) return IDQN_OK;
+  if (h->h_vact) CK(cudaFreeHost(h->h_vact));
+  if (h->h_vout) CK(cudaFreeHost(h->h_vout));
+  h->h_vact = nullptr, h->h_vout = nullptr, h->vact_chunks = 0;
+  CK(cudaMallocHost(&h->h_vact, (size_t)chunks * vact_block(h)));
+  CK(cudaMallocHost(&h->h_vout, sizeof(int32_t) * chunks * h->B));
+  h->vact_chunks = chunks;
+  return IDQN_OK;
+}
+
+// the fast path's graph for a chunk of p (a power of two, or B) images: H2D of the staging block, the forward of every
+// online head over images [0, p), act_select_kernel, D2H of the p actions.  Captured against chunk 0's pinned regions;
+// vact_launch re-points the two copies at the chunk it runs.
+static int vact_capture(idqn_handle* h, int slot, int p) {
+  const size_t h2d = vact_states_off(h) + (size_t)p * h->in_elems;
+  void* s0 = h->s;
+  h->s = h->d_vact + vact_states_off(h);  // s2d_input_kernel reads the staged states in place
+  cudaGraph_t g = nullptr;
+  CK(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
+  int rc = cudaMemcpyAsync(h->d_vact, h->h_vact, h2d, cudaMemcpyHostToDevice, h->stream) == cudaSuccess
+               ? enqueue_apply_fast(h, 0, h->K, p) : IDQN_ECUDA;
+  if (!rc) {
+    act_select_kernel<<<(p + 3) / 4, 128, 0, h->stream>>>(h->q, h->A, (const int32_t*)h->d_vact, p, h->d_vout);
+    if (cudaGetLastError() != cudaSuccess ||
+        cudaMemcpyAsync(h->h_vout, h->d_vout, sizeof(int32_t) * p, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess)
+      rc = IDQN_ECUDA;
+  }
+  cudaError_t e = cudaStreamEndCapture(h->stream, &g);
+  h->s = s0;
+  if (rc || e != cudaSuccess) {
+    if (e == cudaSuccess && g) cudaGraphDestroy(g);
+    if (!rc) idqn_set_error("select_actions: graph capture failed: %s", cudaGetErrorString(e));
+    return rc ? rc : IDQN_ECUDA;
+  }
+  size_t n_nodes = 0;
+  CK(cudaGraphGetNodes(g, nullptr, &n_nodes));
+  std::vector<cudaGraphNode_t> nodes(n_nodes);
+  CK(cudaGraphGetNodes(g, nodes.data(), &n_nodes));
+  h->vact_h2d[slot] = h->vact_d2h[slot] = nullptr;
+  for (cudaGraphNode_t nd : nodes) {
+    cudaGraphNodeType t;
+    CK(cudaGraphNodeGetType(nd, &t));
+    if (t != cudaGraphNodeTypeMemcpy) continue;
+    cudaMemcpy3DParms mp;
+    CK(cudaGraphMemcpyNodeGetParams(nd, &mp));
+    (mp.dstPtr.ptr == h->d_vact ? h->vact_h2d : h->vact_d2h)[slot] = nd;
+  }
+  if (!h->vact_h2d[slot] || !h->vact_d2h[slot]) {
+    cudaGraphDestroy(g);
+    REQUIRE(false, "internal: select_actions graph without its two copies");
+  }
+  cudaError_t ei = cudaGraphInstantiate(&h->vact_exec[slot], g, 0);
+  if (ei != cudaSuccess) {
+    cudaGraphDestroy(g);
+    CK(ei);
+  }
+  h->vact_graph[slot] = g;
+  return IDQN_OK;
+}
+
+static int vact_launch(idqn_handle* h, int64_t chunk, int p) {
+  int slot = 0;
+  while ((1 << slot) < p) ++slot;
+  if (!h->vact_exec[slot]) {
+    int rc = vact_capture(h, slot, p);
+    if (rc) return rc;
+  }
+  const size_t h2d = vact_states_off(h) + (size_t)p * h->in_elems;
+  CK(cudaGraphExecMemcpyNodeSetParams1D(h->vact_exec[slot], h->vact_h2d[slot], h->d_vact,
+                                        h->h_vact + chunk * vact_block(h), h2d, cudaMemcpyHostToDevice));
+  CK(cudaGraphExecMemcpyNodeSetParams1D(h->vact_exec[slot], h->vact_d2h[slot], h->h_vout + chunk * h->B, h->d_vout,
+                                        sizeof(int32_t) * p, cudaMemcpyDeviceToHost));
+  CK(cudaGraphLaunch(h->vact_exec[slot], h->stream));
+  return IDQN_OK;
+}
+
+// N x select_action (utils.py:8-15, idqn.py:126-131): env i draws with key (keys[2i], keys[2i+1]) exactly what
+// idqn_select_action draws; the greedy ones are answered by one device pass per chunk of up to B environments.
+extern "C" int idqn_select_actions(idqn_handle* h, const void* states, int u8, int n, const uint32_t* keys, int n_actions,
+                                   float epsilon, int32_t* actions, int32_t* info) {
+  REQUIRE(h, "null handle");
+  REQUIRE(n >= 0, "select_actions: n = %d < 0", n);
+  REQUIRE(n_actions > 0, "select_actions: n_actions = %d <= 0", n_actions);
+  if (n == 0) return IDQN_OK;
+  REQUIRE(states && keys && actions, "null argument");
+  std::vector<int32_t> head(n), code(n);
+  int n_greedy = 0;
+  for (int i = 0; i < n; ++i) {
+    uint32_t ks[6];
+    tf_split(keys[2 * i], keys[2 * i + 1], 3, ks);
+    const bool explore = tf_uniform(ks[0], ks[1]) <= epsilon;
+    head[i] = tf_randint(ks[4], ks[5], 0, h->K);
+    if (info) info[2 * i] = explore ? 1 : 0, info[2 * i + 1] = head[i];
+    if (explore) actions[i] = tf_randint(ks[2], ks[3], 0, n_actions);
+    code[i] = explore ? -1 - actions[i] : head[i];
+    n_greedy += !explore;
+  }
+  if (!n_greedy) return IDQN_OK;  // no device work at all when every environment explores
+  CK(cudaSetDevice(h->cfg.device));
+  const size_t esz = u8 ? 1 : 4, sbytes = (size_t)h->in_elems * esz;
+  const int B = h->B;
+  int rc;
+  if (apply_fast_ok(h, IDQN_ONLINE, u8) && !(h->cfg.flags & IDQN_F_NO_GRAPH)) {
+    const int64_t chunks = (n + B - 1) / B;
+    if ((rc = vact_reserve(h, chunks))) return rc;
+    if ((rc = refresh_planes(h))) return rc;  // outside the capture, as in idqn_best_action
+    for (int64_t c = 0; c < chunks; ++c) {
+      const int i0 = (int)(c * B), m = std::min(B, n - i0);
+      bool any = false;
+      for (int j = 0; j < m; ++j) any |= code[i0 + j] >= 0;
+      if (!any) continue;
+      int p = 1;
+      while (p < m) p <<= 1;
+      p = std::min(p, B);
+      uint8_t* blk = h->h_vact + c * vact_block(h);
+      int32_t* bc = (int32_t*)blk;
+      uint8_t* bs = blk + vact_states_off(h);
+      for (int j = 0; j < p; ++j) bc[j] = j >= m ? -1 : code[i0 + j] >= 0 ? code[i0 + j] * B + j : code[i0 + j];
+      memcpy(bs, (const uint8_t*)states + (size_t)i0 * sbytes, (size_t)m * sbytes);
+      memset(bs + (size_t)m * sbytes, 0, (size_t)(p - m) * sbytes);  // padding: zero images
+      if ((rc = vact_launch(h, c, p))) return rc;
+    }
+    CK(cudaStreamSynchronize(h->stream));
+    for (int i = 0; i < n; ++i)
+      if (code[i] >= 0) actions[i] = h->h_vout[i];  // chunk c's actions sit at h_vout + c * B
+    return IDQN_OK;
+  }
+  // generic path: the greedy states grouped by head (pinned, in chunks of B), enqueue_apply of that head per chunk, then
+  // act_select_kernel over its q rows
+  std::vector<int> order;
+  order.reserve(n_greedy);
+  for (int k = 0; k < h->K; ++k)
+    for (int i = 0; i < n; ++i)
+      if (code[i] == k) order.push_back(i);
+  const int64_t blocks = ((int64_t)n_greedy * sbytes + vact_block(h) - 1) / vact_block(h);
+  if ((rc = vact_reserve(h, std::max<int64_t>(blocks, (n_greedy + B - 1) / B)))) return rc;
+  for (int j = 0; j < n_greedy; ++j)
+    memcpy(h->h_vact + (size_t)j * sbytes, (const uint8_t*)states + (size_t)order[j] * sbytes, sbytes);
+  for (int j0 = 0; j0 < n_greedy;) {
+    const int k = code[order[j0]];
+    int m = 0;
+    while (j0 + m < n_greedy && m < B && code[order[j0 + m]] == k) ++m;
+    CK(cudaMemcpyAsync(h->s, h->h_vact + (size_t)j0 * sbytes, (size_t)m * sbytes, cudaMemcpyHostToDevice, h->stream));
+    if ((rc = enqueue_apply(h, IDQN_ONLINE, k, u8, m))) return rc;
+    act_select_kernel<<<(m + 3) / 4, 128, 0, h->stream>>>(h->q, h->A, nullptr, m, h->d_vout);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h->h_vout + j0, h->d_vout, sizeof(int32_t) * m, cudaMemcpyDeviceToHost, h->stream));
+    j0 += m;
+  }
+  CK(cudaStreamSynchronize(h->stream));
+  for (int j = 0; j < n_greedy; ++j) actions[order[j]] = h->h_vout[j];
+  return IDQN_OK;
 }
 
 // IDQN_F_TIMELINE: per-CTA stamps (entry, first operand landed, last MMA committed, exit; ns) of the kernel in timeline slot

@@ -27,7 +27,8 @@ import numpy as np
 
 from .. import _prng
 from .. import checkpoint as ckpt
-from ..sample_collection.utils import collect_single_sample
+from ..sample_collection.replay_buffer import TransitionElement
+from ..sample_collection.utils import collect_single_sample, select_actions
 
 
 def linear_schedule(init_value: float, end_value: float, transition_steps: int):
@@ -105,6 +106,89 @@ def train(key, p: dict, agent, env, rb):
                 "key": [int(k) for k in _prng.as_key(key)],
                 "returns": episode_returns_per_epoch, "lengths": episode_lengths_per_epoch})
             ckpt.commit(root, str(idx_epoch), keep=rb._checkpoint_duration)
+    return episode_returns_per_epoch, episode_lengths_per_epoch
+
+
+def train_vectorized(key, p: dict, agent, envs, rb):
+    """``train`` over N environments that act together: each iteration draws N + 1 keys, chooses all N actions in one
+    ``select_actions`` call, then steps the environments in order, each step followed by ``train``'s body (replay ``add``
+    into that environment's accumulator, reset on episode end, the learner past ``n_initial_samples``).  The learner
+    still runs after every environment step, so ``update_to_data`` and the target schedule count environment steps.
+
+    ``rb`` must have been built with ``n_envs=len(envs)``.  With one environment this is ``train`` exactly (the same
+    keys, actions, epochs, returns and logs).  With more, an epoch ends at the first iteration boundary after at least
+    ``n_training_steps_per_epoch`` environment steps; an episode's return and length go to the epoch in which it ended,
+    and episodes still running carry over.  ``p["checkpoint_dir"]`` is refused: environments cannot be saved mid-episode."""
+    if p.get("checkpoint_dir") is not None:
+        raise ValueError("train_vectorized does not checkpoint (environments cannot be saved mid-episode): "
+                         "remove p['checkpoint_dir']")
+    n_envs = len(envs)
+    if n_envs < 1 or getattr(rb, "_n_envs", 1) != n_envs:
+        raise ValueError(f"train_vectorized needs a ReplayBuffer with n_envs={n_envs}, got {getattr(rb, '_n_envs', 1)}")
+    epsilon_schedule = linear_schedule(1.0, p["epsilon_end"], p["epsilon_duration"])
+    log = p["wandb"].log if p.get("wandb") is not None else (lambda d: None)
+    single = n_envs == 1
+
+    n_training_steps = 0
+    for env in envs:
+        env.reset()
+    # one environment: train's lists (the running episode is the last entry); several: finished episodes only
+    episode_returns_per_epoch = [[0]] if single else [[]]
+    episode_lengths_per_epoch = [[0]] if single else [[]]
+    running_return, running_length = [0.0] * n_envs, [0] * n_envs
+
+    for idx_epoch in range(p["n_epochs"]):
+        n_training_steps_epoch = 0
+        has_reset = False
+
+        while n_training_steps_epoch < p["n_training_steps_per_epoch"] or (single and not has_reset):
+            key, *env_keys = _prng.split(key, n_envs + 1)
+            actions = select_actions(agent.best_action, agent.params, [env.state for env in envs], env_keys,
+                                     envs[0].n_actions, epsilon_schedule, n_training_steps)
+            for i, env in enumerate(envs):
+                action = int(actions[i])
+                obs = env.observation
+                reward, absorbing = env.step(action)
+                has_reset = absorbing or env.n_steps >= p["horizon"]
+                rb.add(TransitionElement(observation=obs, action=action,
+                                         reward=reward if rb._clipping is None else rb._clipping(reward),
+                                         is_terminal=absorbing, episode_end=has_reset), env=i)
+                if has_reset:
+                    env.reset()
+
+                n_training_steps_epoch += 1
+                n_training_steps += 1
+
+                if single:
+                    episode_returns_per_epoch[idx_epoch][-1] += reward
+                    episode_lengths_per_epoch[idx_epoch][-1] += 1
+                    if has_reset and n_training_steps_epoch < p["n_training_steps_per_epoch"]:
+                        episode_returns_per_epoch[idx_epoch].append(0)
+                        episode_lengths_per_epoch[idx_epoch].append(0)
+                else:
+                    running_return[i] += reward
+                    running_length[i] += 1
+                    if has_reset:
+                        episode_returns_per_epoch[idx_epoch].append(running_return[i])
+                        episode_lengths_per_epoch[idx_epoch].append(running_length[i])
+                        running_return[i], running_length[i] = 0.0, 0
+
+                if n_training_steps > p["n_initial_samples"]:
+                    agent.update_online_params(n_training_steps, rb)
+                    target_updated, logs = agent.update_target_params(n_training_steps)
+                    if target_updated:
+                        log({"n_training_steps": n_training_steps, **logs})
+
+        finished = episode_returns_per_epoch[idx_epoch]
+        avg_return = np.mean(finished) if finished else float("nan")  # several environments: maybe none ended
+        avg_length_episode = np.mean(episode_lengths_per_epoch[idx_epoch]) if finished else float("nan")
+        log({"epoch": idx_epoch, "n_training_steps": n_training_steps, "avg_return": avg_return,
+             "avg_length_episode": avg_length_episode})
+        if idx_epoch < p["n_epochs"] - 1:
+            episode_returns_per_epoch.append([0] if single else [])
+            episode_lengths_per_epoch.append([0] if single else [])
+        if p.get("save") is not None:
+            p["save"](p, episode_returns_per_epoch, episode_lengths_per_epoch, agent.get_model())
     return episode_returns_per_epoch, episode_lengths_per_epoch
 
 

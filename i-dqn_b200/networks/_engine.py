@@ -367,6 +367,26 @@ class Engine:
                                             float(epsilon), C.byref(out), L.ptr(info)))
         return int(out.value), bool(info[0]), int(info[1])
 
+    def select_actions(self, states, keys, n_actions: int, epsilon: float):
+        """``select_action`` for N environments in one C call: env i draws with ``keys[i]`` and the greedy ones share one
+        device pass per chunk of up to B states.  Returns (actions int32[N], explored bool[N], heads int32[N])."""
+        from .. import _prng
+        ks = np.ascontiguousarray([_prng.as_key(k) for k in keys], np.uint32).reshape(-1, 2)
+        n = len(ks)
+        x = np.asarray(states)
+        u8 = x.dtype == np.uint8
+        if not u8 and self.architecture_type == "cnn":
+            xu = x.astype(np.uint8)  # atari.py:43-45 hands over float32 frames holding 0..255
+            if np.array_equal(xu, x):
+                x, u8 = xu, True
+        x = np.ascontiguousarray(x, dtype=np.uint8 if u8 else np.float32)
+        if x.size != n * self.in_elems:
+            raise ValueError(f"states have {x.size} elements, expected {n} x {self.in_elems} for {n} keys")
+        out, info = np.zeros(n, np.int32), np.zeros((n, 2), np.int32)
+        L.check(self.lib.idqn_select_actions(self.h, L.ptr(x), int(u8), n, L.ptr(ks), int(n_actions), float(epsilon),
+                                             L.ptr(out), L.ptr(info)))
+        return out, info[:, 0].astype(bool), info[:, 1].copy()
+
     def mark_head_planes_dirty(self, which: int, head: int) -> None:
         """One head of an arena was rewritten behind the library's back (neighbour exchange): rebuild its planes."""
         L.check(self.lib.idqn_mark_head_planes_dirty(self.h, which, int(head)))

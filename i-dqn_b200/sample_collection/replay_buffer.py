@@ -235,7 +235,10 @@ class ReplayBuffer:
         *,
         device: int = 0,
         frame_store: bool = False,
+        n_envs: int = 1,
     ):
+        if int(n_envs) != n_envs or n_envs < 1:
+            raise ValueError(f"n_envs must be a positive integer, got {n_envs!r}")
         self.add_count = 0
         self._max_capacity = max_capacity
         self._compress = compress  # accepted for signature parity; HBM slots hold raw bytes
@@ -249,21 +252,26 @@ class ReplayBuffer:
         self._device = device
         self._store: Optional[_DeviceStore] = None
         self._memory = _MemoryView(self)
-        self._trajectory: "collections.deque[TransitionElement]" = collections.deque(
-            maxlen=self._update_horizon + self._stack_size)
+        # one n-step / frame-stack accumulator per environment (``add(..., env=i)``); ``_trajectory`` is environment 0's
+        self._n_envs = int(n_envs)
+        self._trajectories: "list[collections.deque[TransitionElement]]" = [
+            collections.deque(maxlen=self._update_horizon + self._stack_size) for _ in range(self._n_envs)]
+        self._trajectory = self._trajectories[0]
         self._frame_store = frame_store
         if frame_store:
-            # frame id of each trajectory entry once an emitted element has referred to it (None before)
-            self._frame_ids: "collections.deque[Optional[int]]" = collections.deque(maxlen=self._trajectory.maxlen)
+            # frame id of each trajectory entry once an emitted element has referred to it (None before), per environment
+            self._env_frame_ids: "list[collections.deque[Optional[int]]]" = [
+                collections.deque(maxlen=self._trajectory.maxlen) for _ in range(self._n_envs)]
+            self._frame_ids = self._env_frame_ids[0]
             self._next_frame_id = 0
             # (key, smallest frame id) of live elements with that id increasing: the front is the smallest of all
             self._live_min: "collections.deque[tuple[int, int]]" = collections.deque()
 
     # ---- n-step / frame-stack accumulator (replay_buffer.py:103-200) ---------------------------------
-    def _window(self) -> Optional[tuple[int, list[int]]]:
-        """The element the trajectory emits now, as (pivot, trajectory index of each of the 2 * stack stack positions:
-        state, then next_state; -1 = zero), or None."""
-        traj, n, stack = self._trajectory, self._update_horizon, self._stack_size
+    def _window(self, env: int = 0) -> Optional[tuple[int, list[int]]]:
+        """The element environment ``env``'s trajectory emits now, as (pivot, trajectory index of each of the 2 * stack
+        stack positions: state, then next_state; -1 = zero), or None."""
+        traj, n, stack = self._trajectories[env], self._update_horizon, self._stack_size
         length = len(traj)
         newest = traj[-1]
         if not (length > n or (length > 1 and newest.is_terminal)):
@@ -276,16 +284,16 @@ class ReplayBuffer:
         next_state = [max(length - stack + pos, -1) for pos in range(stack)]
         return pivot, state + next_state
 
-    def _scalars(self, pivot: int) -> tuple[Any, float, bool]:
-        traj, n = self._trajectory, self._update_horizon
+    def _scalars(self, pivot: int, env: int = 0) -> tuple[Any, float, bool]:
+        traj, n = self._trajectories[env], self._update_horizon
         ret = 0.0
         for t in range(pivot, min(pivot + n, len(traj))):  # discounted n-step return (:153-165)
             ret += traj[t].reward * (self._gamma ** (t - pivot))
         return traj[pivot].action, ret, traj[-1].is_terminal
 
-    def _make_replay_element(self, window) -> ReplayElement:
+    def _make_replay_element(self, window, env: int = 0) -> ReplayElement:
         pivot, positions = window
-        traj, stack = self._trajectory, self._stack_size
+        traj, stack = self._trajectories[env], self._stack_size
         frame = np.asarray(traj[-1].observation)
         state = np.zeros(frame.shape + (stack,), frame.dtype)
         next_state = np.zeros(frame.shape + (stack,), frame.dtype)
@@ -295,40 +303,50 @@ class ReplayBuffer:
                 state[..., pos] = traj[t_state].observation
             if t_next >= 0:
                 next_state[..., pos] = traj[t_next].observation
-        action, ret, terminal = self._scalars(pivot)
+        action, ret, terminal = self._scalars(pivot, env)
         return ReplayElement(state=state, action=action, reward=ret, next_state=next_state, is_terminal=terminal,
                              episode_end=terminal)
 
-    def _windows(self, transition: TransitionElement) -> Iterator[tuple[int, list[int]]]:
-        self._trajectory.append(transition)
+    def _windows(self, transition: TransitionElement, env: int = 0) -> Iterator[tuple[int, list[int]]]:
+        traj = self._trajectories[env]
+        traj.append(transition)
         if self._frame_store:
-            self._frame_ids.append(None)
+            self._env_frame_ids[env].append(None)
         if transition.is_terminal:  # drain: one element per remaining start frame (:189-194)
-            while (window := self._window()) is not None:
+            while (window := self._window(env)) is not None:
                 yield window
-                self._trajectory.popleft()
+                traj.popleft()
                 if self._frame_store:
-                    self._frame_ids.popleft()
-            self._clear_trajectory()
+                    self._env_frame_ids[env].popleft()
+            self._clear_trajectory(env)
         else:
-            if (window := self._window()) is not None:
+            if (window := self._window(env)) is not None:
                 yield window
             if transition.episode_end:  # truncation (:199-200)
-                self._clear_trajectory()
+                self._clear_trajectory(env)
 
-    def _clear_trajectory(self) -> None:
-        self._trajectory.clear()
+    def _clear_trajectory(self, env: int = 0) -> None:
+        self._trajectories[env].clear()
         if self._frame_store:
-            self._frame_ids.clear()
+            self._env_frame_ids[env].clear()
 
-    def accumulate(self, transition: TransitionElement) -> Iterable[ReplayElement]:
-        for window in self._windows(transition):
-            yield self._make_replay_element(window)
+    def _check_env(self, env) -> int:
+        if not isinstance(env, (int, np.integer)) or not 0 <= env < self._n_envs:
+            raise ValueError(f"env={env!r} is not one of this buffer's {self._n_envs} environments")
+        return int(env)
+
+    def accumulate(self, transition: TransitionElement, env: int = 0) -> Iterable[ReplayElement]:
+        env = self._check_env(env)
+        for window in self._windows(transition, env):
+            yield self._make_replay_element(window, env)
 
     # ---- frame store bookkeeping ----------------------------------------------------------------------
     # Invariant: every frame id a live element or the trajectory refers to lies in [next id - n_frames, next id), so
     # writing id f into ring slot f % n_frames never overwrites a frame still in use.  An id leaves that set for good
     # (the trajectory only drops entries, elements are evicted in FIFO order), so its smallest member never decreases.
+    # With several environments the set holds every environment's trajectory ids; a newly assigned id is still the
+    # largest of all, so the argument holds.  An environment that is never stepped again keeps its trajectory's frames
+    # in use for good: the ring grows to hold them next to everything written after them.
     _frame_store_type = _FrameStore  # anything with put_frame / put_element / grow / n_frames (a host model in tests)
 
     def _open_frame_store(self, frame: np.ndarray) -> _FrameStore:
@@ -337,7 +355,7 @@ class ReplayBuffer:
         return self._frame_store_type(cap, frame.shape, frame.dtype, stack, n_frames, self._device)
 
     def _lowest_frame_in_use(self) -> int:
-        ids = [f for f in self._frame_ids if f is not None]
+        ids = [f for frame_ids in self._env_frame_ids for f in frame_ids if f is not None]
         if self._live_min:
             ids.append(self._live_min[0][1])
         return min(ids, default=self._next_frame_id)
@@ -354,15 +372,16 @@ class ReplayBuffer:
         self._next_frame_id = f + 1
         return f
 
-    def _add_frames(self, key: int, window) -> None:
+    def _add_frames(self, key: int, window, env: int = 0) -> None:
         pivot, positions = window
+        traj, frame_ids = self._trajectories[env], self._env_frame_ids[env]
         while self._live_min and self._live_min[0][0] <= key - self._max_capacity:  # the element `key` replaces
             self._live_min.popleft()
         for t in sorted({t for t in positions if t >= 0}):  # ids in trajectory order, on first use
-            if self._frame_ids[t] is None:
-                self._frame_ids[t] = self._new_frame_id(self._trajectory[t].observation)
-        ids = [self._frame_ids[t] if t >= 0 else -1 for t in positions]
-        action, ret, terminal = self._scalars(pivot)
+            if frame_ids[t] is None:
+                frame_ids[t] = self._new_frame_id(traj[t].observation)
+        ids = [frame_ids[t] if t >= 0 else -1 for t in positions]
+        action, ret, terminal = self._scalars(pivot, env)
         self._store.put_element(key % self._max_capacity, ids, action, ret, terminal, terminal)
         smallest = min(f for f in ids if f >= 0)
         while self._live_min and self._live_min[-1][1] >= smallest:
@@ -370,15 +389,18 @@ class ReplayBuffer:
         self._live_min.append((key, smallest))
 
     # ---- add / sample / update (replay_buffer.py:202-237) -----------------------------------------------
-    def add(self, transition: TransitionElement, **kwargs: Any) -> None:
-        for window in self._windows(transition):
+    def add(self, transition: TransitionElement, *, env: int = 0, **kwargs: Any) -> None:
+        """Add a transition of environment ``env`` (one of ``n_envs``); elements get keys in the order they are emitted,
+        whichever environment emits them.  ``kwargs`` go to the sampler."""
+        env = self._check_env(env)
+        for window in self._windows(transition, env):
             key = ReplayItemID(self.add_count)
             if self._frame_store:
                 if self._store is None:
                     self._store = self._open_frame_store(np.asarray(transition.observation))
-                self._add_frames(key, window)
+                self._add_frames(key, window, env)
             else:
-                element = self._make_replay_element(window)
+                element = self._make_replay_element(window, env)
                 if self._store is None:
                     self._store = _DeviceStore(self._max_capacity, np.shape(element.state),
                                                np.asarray(element.state).dtype, self._device)
@@ -434,10 +456,17 @@ class ReplayBuffer:
     _DIGESTS = ("state/frames", "next_state/rows", "action", "reward", "terminal", "episode_end")
 
     def _config(self) -> dict:
-        return {"max_capacity": int(self._max_capacity), "stack_size": int(self._stack_size),
-                "update_horizon": int(self._update_horizon), "gamma": float(self._gamma),
-                "batch_size": int(self._batch_size), "frame_store": bool(self._frame_store),
-                "sampler": type(self._sampling_distribution).__name__}
+        config = {"max_capacity": int(self._max_capacity), "stack_size": int(self._stack_size),
+                  "update_horizon": int(self._update_horizon), "gamma": float(self._gamma),
+                  "batch_size": int(self._batch_size), "frame_store": bool(self._frame_store),
+                  "sampler": type(self._sampling_distribution).__name__}
+        if self._n_envs != 1:  # a checkpoint without the key is of one environment
+            config["n_envs"] = self._n_envs
+        return config
+
+    @staticmethod
+    def _trajectory_file(env: int, field: str) -> str:
+        return f"trajectory_{field}.npy" if env == 0 else f"trajectory{env}_{field}.npy"
 
     def _slot_files(self):
         return ("rows" if self._frame_store else "state", "next_state", "action", "reward", "terminal", "episode_end")
@@ -446,16 +475,22 @@ class ReplayBuffer:
         """Write this buffer into ``directory`` (created if missing).  Waits for learner steps still reading the store."""
         os.makedirs(directory, exist_ok=True)
         join = lambda name: os.path.join(directory, name)
-        traj = list(self._trajectory)
-        meta = {"config": self._config(), "add_count": int(self.add_count), "trajectory": len(traj), "store": None}
-        if traj:
-            np.save(join("trajectory_observation.npy"), np.stack([np.asarray(t.observation) for t in traj]))
-            np.save(join("trajectory_action.npy"), np.asarray([int(t.action) for t in traj], np.int64))
-            np.save(join("trajectory_reward.npy"), np.asarray([float(t.reward) for t in traj], np.float64))
-            np.save(join("trajectory_flags.npy"),
-                    np.asarray([(bool(t.is_terminal), bool(t.episode_end)) for t in traj], np.uint8).reshape(-1, 2))
+        meta = {"config": self._config(), "add_count": int(self.add_count), "trajectory": len(self._trajectory),
+                "store": None}
+        if self._n_envs != 1:  # environment i's accumulator in trajectory{i}_*.npy (environment 0's as with one)
+            meta["trajectories"] = [len(t) for t in self._trajectories]
+        for env, traj in enumerate(self._trajectories):
+            if traj:
+                name = lambda field: join(self._trajectory_file(env, field))
+                np.save(name("observation"), np.stack([np.asarray(t.observation) for t in traj]))
+                np.save(name("action"), np.asarray([int(t.action) for t in traj], np.int64))
+                np.save(name("reward"), np.asarray([float(t.reward) for t in traj], np.float64))
+                np.save(name("flags"),
+                        np.asarray([(bool(t.is_terminal), bool(t.episode_end)) for t in traj], np.uint8).reshape(-1, 2))
         if self._frame_store:
             meta["frame_ids"] = [-1 if f is None else int(f) for f in self._frame_ids]
+            if self._n_envs != 1:
+                meta["env_frame_ids"] = [[-1 if f is None else int(f) for f in ids] for ids in self._env_frame_ids]
             meta["next_frame_id"] = int(self._next_frame_id)
             meta["live_min"] = [[int(k), int(f)] for k, f in self._live_min]
         st = self._store
@@ -496,20 +531,23 @@ class ReplayBuffer:
         against the saved digests on the device (ValueError on a mismatch; the buffer is then unusable)."""
         join = lambda name: os.path.join(directory, name)
         meta = ckpt.read_json(join("replay.json"))
-        if self.add_count != 0 or self._store is not None or self._trajectory:
+        if self.add_count != 0 or self._store is not None or any(self._trajectories):
             raise ValueError("ReplayBuffer.load needs a buffer nothing has been added to")
-        for k, v in self._config().items():
-            if meta["config"][k] != v:
-                raise ValueError(f"replay checkpoint has {k}={meta['config'][k]!r}, this buffer {v!r}")
-        if meta["trajectory"]:
-            obs = np.load(join("trajectory_observation.npy"))
-            act, rew = np.load(join("trajectory_action.npy")), np.load(join("trajectory_reward.npy"))
-            flags = np.load(join("trajectory_flags.npy"))
-            for t in range(meta["trajectory"]):
-                self._trajectory.append(TransitionElement(obs[t], int(act[t]), float(rew[t]), bool(flags[t, 0]),
-                                                          bool(flags[t, 1])))
+        saved = {"n_envs": 1, **meta["config"]}
+        for k, v in {"n_envs": 1, **self._config()}.items():
+            if saved[k] != v:
+                raise ValueError(f"replay checkpoint has {k}={saved[k]!r}, this buffer {v!r}")
+        for env, length in enumerate(meta.get("trajectories", [meta["trajectory"]])):
+            if length:
+                name = lambda field: join(self._trajectory_file(env, field))
+                obs, act, rew = np.load(name("observation")), np.load(name("action")), np.load(name("reward"))
+                flags = np.load(name("flags"))
+                for t in range(length):
+                    self._trajectories[env].append(TransitionElement(obs[t], int(act[t]), float(rew[t]),
+                                                                     bool(flags[t, 0]), bool(flags[t, 1])))
         if self._frame_store:
-            self._frame_ids.extend(None if f < 0 else f for f in meta["frame_ids"])
+            for ids, saved_ids in zip(self._env_frame_ids, meta.get("env_frame_ids", [meta["frame_ids"]])):
+                ids.extend(None if f < 0 else f for f in saved_ids)
             self._next_frame_id = meta["next_frame_id"]
             self._live_min.extend((k, f) for k, f in meta["live_min"])
         sm = meta["store"]

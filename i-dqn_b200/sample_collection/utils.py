@@ -3,6 +3,8 @@
 reference training loop runs unchanged against this package.  PRNG semantics: ``idqn_b200._prng``."""
 from __future__ import annotations
 
+import numpy as np
+
 from .. import _prng
 from .replay_buffer import ReplayBuffer, TransitionElement
 
@@ -18,6 +20,22 @@ def select_action(best_action_fn, params, state, key, n_actions, epsilon_fn, n_t
     if _prng.uniform(uniform_key) <= epsilon_fn(n_training_steps):  # utils.py:12
         return _prng.randint(action_key, 0, n_actions)
     return best_action_fn(params, state, key=kwargs_key)  # only the taken branch is evaluated
+
+
+def select_actions(best_action_fn, params, states, keys, n_actions, epsilon_fn, n_training_steps) -> np.ndarray:
+    """``select_action`` for N environments: ``out[i] == select_action(best_action_fn, params, states[i], keys[i], ...)``.
+    For the agent's own live online parameters (iDQN, and DQN, whose head draw ``randint(., 0, 1)`` is always 0) the
+    draws and the greedy forward passes of all N environments run in one call into the library; anything else is the
+    per-environment loop."""
+    agent = getattr(best_action_fn, "__self__", None)
+    engine = getattr(agent, "_engine", None)
+    if len(states) != len(keys):
+        raise ValueError(f"{len(states)} states but {len(keys)} keys")
+    if engine is not None and getattr(params, "_engine_ref", lambda: None)() is engine and getattr(params, "_which", None) == 0 \
+            and (engine.K == 1 if getattr(agent, "_squeeze", False) else getattr(agent, "n_networks", 0) == engine.K):
+        return engine.select_actions(states, keys, n_actions, epsilon_fn(n_training_steps))[0]
+    return np.asarray([select_action(best_action_fn, params, s, k, n_actions, epsilon_fn, n_training_steps)
+                       for s, k in zip(states, keys)], np.int32).reshape(len(keys))
 
 
 def collect_single_sample(key, env, agent, rb: ReplayBuffer, p, epsilon_schedule, n_training_steps: int):

@@ -193,6 +193,15 @@ int idqn_best_action(idqn_handle* h, int which, int head, const void* state_host
  * key0/key1: the uint32[2] jax key; info (optional, int32[2]): {explored, head}. */
 int idqn_select_action(idqn_handle* h, const void* state_host, int state_is_u8, uint32_t key0, uint32_t key1,
                        int n_actions, float epsilon, int32_t* action, int32_t* info);
+/* N independent select_action draws (slimdqn/sample_collection/utils.py:8-15, head draw idqn.py:126-131) in ONE call:
+ * env i makes exactly the draws of idqn_select_action with the key (keys[2i], keys[2i+1]).  states: n * in_elems values
+ * (uint8 if state_is_u8, else float32); actions: [n]; info (optional): [n][2] = {explored, head}.  No device work when
+ * every environment explores; otherwise, at Atari shapes with uint8 states, one CUDA-graph launch per chunk of up to
+ * batch_size environments (the online heads' forward of the chunk's states and the per-environment argmax of the drawn
+ * head's Q row) and one host synchronisation at the end.  Q rows are bit-identical to idqn_best_action's.  Ordered
+ * after every learning step enqueued before it.  IDQN_EINVAL for n < 0 or n_actions <= 0. */
+int idqn_select_actions(idqn_handle* h, const void* states_host, int state_is_u8, int n, const uint32_t* keys,
+                        int n_actions, float epsilon, int32_t* actions, int32_t* info);
 /* the draws themselves (tests / host mirrors): what = 0 split(key, a) -> out[2a]; 1 uniform(key) -> float32 bits in out[0];
  * 2 randint(key, (), a, b) -> out[0] */
 int idqn_prng(int what, uint32_t key0, uint32_t key1, int32_t a, int32_t b, uint32_t* out);
