@@ -15,7 +15,7 @@ struct ImgHost {
   // weight-streaming kernels of the big Dense layer (dense_stream.cuh)
   int dense_on;
   alignas(64) CUtensorMap fmapWf[2], fmapWd, dmapX[2], dmapDy[2];  // fp32 Dense_0 kernel: fwd boxes {128 o, 64 i} of the online / target arena, dgrad boxes {64 o, 128 i} (online)
-  alignas(64) CUtensorMap wmapX[2], wmapP[3];  // dense_wgrad_tma.cuh: x planes {32 i, 32 b}; fp32 W / mu / nu {256 o, 8 i}
+  alignas(64) CUtensorMap wmapX[2], wmapP[3];  // dense_wgrad_tma.cuh: x planes {16 i, 32 b}; fp32 W / mu / nu {256 o, 8 i}
   int wgrad_tma_on;
   dense::Args dfwd, ddg;
   float* dpart;
@@ -384,12 +384,12 @@ static int img_setup(idqn_handle* h) {
       H->wgrad_tma_on = O == dwt::CB * dwt::TO && I % dwt::TM == 0 && dense.b_off == dense.w_off + (int64_t)I * O;
       if (H->wgrad_tma_on) {
         for (int pl = 0; pl < 2; ++pl) {
-          // x planes as the N-side operand: boxes {32 i, 32 b} (64-byte rows); dy planes as the M side: dmapDy {64 o, 32 b}
+          // x planes as the N-side operand: boxes {16 i, 32 b} (32-byte rows, SWIZZLE_32B); dy^T goes to TMEM from global
           const __nv_bfloat16* xb = (pl ? h->act_lo : h->act_hi) + prev.act_off;
           const uint64_t xdims[3] = {(uint64_t)I, (uint64_t)B, (uint64_t)2 * K};
           const uint64_t xstr[2] = {(uint64_t)I * 2, (uint64_t)h->act_stride * 2};
           const uint32_t xbox[3] = {(uint32_t)dwt::TN, (uint32_t)B, 1};
-          REQUIRE(tma::encode_bf16(&H->wmapX[pl], xb, 3, xdims, xstr, xbox, 64), "tensor map dense x (wgrad)");
+          REQUIRE(tma::encode_bf16(&H->wmapX[pl], xb, 3, xdims, xstr, xbox, 32), "tensor map dense x (wgrad)");
         }
         float* arenas[3] = {h->online, h->mu, h->nu};
         for (int a = 0; a < 3; ++a) {
@@ -644,6 +644,7 @@ static int dense_wgrad_launch(idqn_handle* h, int tile0, int ntiles, bool keep_g
   a.count = h->count;
   a.lr = h->cfg.learning_rate, a.b1 = 0.9f, a.b2 = 0.999f, a.eps = h->cfg.adam_eps;
   a.grad = keep_grads ? h->grad : nullptr;
+  a.dyh = h->dact_hi + l.act_off, a.dyl = h->dact_lo + l.act_off, a.dystride = h->act_stride;
   // measured: 98.6 us with the default policy for the fp32 streams, 100.8 us with evict_first
   static const int sp = getenv("IDQN_L2_STREAM") ? atoi(getenv("IDQN_L2_STREAM")) : 0;
   a.stream_policy = sp == 0 ? tma::L2_EVICT_NORMAL : (sp == 2 ? tma::L2_EVICT_LAST : tma::L2_EVICT_FIRST);
@@ -652,7 +653,7 @@ static int dense_wgrad_launch(idqn_handle* h, int tile0, int ntiles, bool keep_g
   const int grid = std::min(a.heads * a.ntiles, h->sm_avail);
   CK(img_set_smem(dwt::dense_wgrad_adam_kernel, dwt::SMEM_TOTAL));
   CK(launch_pdl(0, dwt::dense_wgrad_adam_kernel, dim3(grid), dim3(dwt::NTHREADS), dwt::SMEM_TOTAL, h->stream, H->wmapX[0],
-                H->wmapX[1], H->dmapDy[0], H->dmapDy[1], H->wmapP[0], H->wmapP[1], H->wmapP[2], a));
+                H->wmapX[1], H->wmapP[0], H->wmapP[1], H->wmapP[2], a));
   CK(cudaGetLastError());
   mark(h, "dense_wgrad_adam_L%d", IDQN_IMG_LAYERS);
   return IDQN_OK;

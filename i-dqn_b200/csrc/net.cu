@@ -1056,7 +1056,7 @@ static int launch_adam_ranges(idqn_handle* h, int64_t off_a, int64_t len_a, bool
 static int dense_update_ctas(const idqn_handle* h) {
   static const int env = getenv("IDQN_WG_OVERLAP") ? atoi(getenv("IDQN_WG_OVERLAP")) : -1;
   if (h->update_ctas_set > 0) return std::min(h->sm_count, h->update_ctas_set - 1);
-  return env >= 0 ? env : (h->K <= 10 ? std::min(h->sm_count, (116 + 13 * h->K) / 2 * h->sm_count / 148) : 0);
+  return env >= 0 ? env : (h->K <= 10 ? std::min(h->sm_count, std::min(80, 54 + 6 * h->K) * h->sm_count / 148) : 0);
 }
 
 // dry = only size the split-K workspace
@@ -1184,10 +1184,11 @@ static int enqueue_learn_step(idqn_handle* h, int x_u8, bool dry = false, int64_
   bool overlapped = false;
   int deferred_t0 = 0;
   static const float overlap_frac = getenv("IDQN_WG_FRAC") ? (float)atof(getenv("IDQN_WG_FRAC")) : 1.0f;
-  // CTAs of the Dense_0 update when it runs next to the conv backward chain instead of after it (0: after): 58 + 6.5 K.
-  // Measured on B200 (tools/r2l.sh / r2n.sh, ms per step, update after the chain -> next to it): K=1 0.122 -> 0.112 at
-  // 64-80 CTAs, K=3 0.208 -> 0.197 at 72-80, K=5 0.295 -> 0.274 at 88, K=8 0.417 -> 0.394 at 88-112; fewer CTAs starve the
-  // update (~52 GB/s per SM), more starve the chain.  IDQN_WG_OVERLAP=<n> overrides, 0 restores the back-to-back order.
+  // CTAs of the Dense_0 update when it runs next to the conv backward chain instead of after it (0: after):
+  // min(80, 54 + 6 K).  Measured on a B200 at 1000 W (tools/k_sweep.py under IDQN_WG_OVERLAP = 0, 56, 64, ..., 104, ms per
+  // step, update after the chain -> best count next to it): K=1 0.125 -> 0.1126 at 56-64 CTAs, K=3 0.210 -> 0.193 at 72,
+  // K=5 0.297 -> 0.267 at 80, K=8 0.415 -> 0.379 at 80; fewer CTAs starve the update (~63 GB/s per SM at 80 CTAs), more
+  // starve the chain.  IDQN_WG_OVERLAP=<n> overrides, 0 restores the back-to-back order.
   const int overlap_ctas = dense_update_ctas(h);
   // idqn_profile_step times the kernels one by one on one stream: same grids as in the graph, so that its per-kernel times
   // (bench.py: kernel_ms, roofline) describe the launches the timed step makes
@@ -2358,7 +2359,7 @@ extern "C" int idqn_cta_timeline(idqn_handle* h, int slot, unsigned long long* o
 extern "C" int idqn_dense_update_ctas(idqn_handle* h) { return h ? dense_update_ctas(h) : 0; }
 
 // n > 0: the Dense_0 update runs on n CTAs next to the conv backward chain; 0: after the chain on every SM; < 0: automatic
-// (58 + 6.5 K).  Call before the first learning step: captured graphs keep the schedule they were captured with.
+// (min(80, 54 + 6 K) on 148 SMs).  Call before the first learning step: captured graphs keep the schedule they were captured with.
 extern "C" int idqn_set_dense_update_ctas(idqn_handle* h, int n) {
   REQUIRE(h, "null handle");
   h->update_ctas_set = n < 0 ? 0 : n + 1;

@@ -109,6 +109,16 @@ __device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, float* v) {
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// 32 lanes x 16 consecutive 32-bit columns: thread i of warp w writes row (32*(w%4) + i); complete after tmem_st_wait()
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* r) {
+  __syncwarp();
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
+      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]),
+      "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ---- descriptors ------------------------------------------------------------------------------------------
 // sm_100 shared-memory matrix descriptor, SWIZZLE_NONE (cute/arch/mma_sm100_desc.hpp: SmemDescriptor)

@@ -75,7 +75,7 @@ __device__ __forceinline__ void st1_planes_hint(__nv_bfloat16* hi, __nv_bfloat16
 }
 
 // UMMA layout types (cute/arch/mma_sm100_desc.hpp: UMMA::LayoutType)
-constexpr uint32_t LT_SW128 = 2, LT_SW64 = 4;
+constexpr uint32_t LT_SW128 = 2, LT_SW64 = 4, LT_SW32 = 6;
 // swizzled shared-memory matrix descriptor; saddr may be any 16-byte aligned address inside a 1024-byte aligned tile
 __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout_type) {
   uint64_t d = 0;
@@ -125,6 +125,21 @@ __device__ __forceinline__ void mma_bf16_split(uint32_t d_tmem, uint32_t a_lo, u
         : "memory");
   }
 }
+// The same with the A operand in tensor memory: M = 128 lanes (row m = lane m), K-major, two bf16 per 32-bit column
+// (element k in the low half of column k / 2), so one K = 16 step reads 8 columns from a_tmem.  idesc: a_major = K.
+template <bool ACC>
+__device__ __forceinline__ void mma_bf16_tmem_a(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_lo, uint32_t b_hi, uint32_t idesc) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      ".reg .b64 db;\n"
+      "setp.ne.u32 p, %5, 0;\n"
+      "mov.b64 db, {%2, %3};\n"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n"
+      "}\n" ::"r"(d_tmem),
+      "r"(a_tmem), "r"(b_lo), "r"(b_hi), "r"(idesc), "n"(ACC ? 1 : 0)
+      : "memory");
+}
 
 // ---- host: tensor-map encoding through the driver entry point (no link-time dependency on libcuda) ----------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -152,7 +167,7 @@ static inline bool encode_f32(CUtensorMap* map, const void* base, int rank, cons
             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-// bf16 tensor, rank <= 4, dims/box innermost first, strides (bytes) for dims 1..rank-1; sw_bytes = 128 or 64
+// bf16 tensor, rank <= 4, dims/box innermost first, strides (bytes) for dims 1..rank-1; sw_bytes = 128, 64 or 32
 static inline bool encode_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides,
                                const uint32_t* box, int sw_bytes) {
   EncodeTiledFn fn = encode_fn();
@@ -161,7 +176,9 @@ static inline bool encode_bf16(CUtensorMap* map, const void* base, int rank, con
   cuuint32_t bx[5], es[5];
   for (int i = 0; i < rank; ++i) gd[i] = dims[i], bx[i] = box[i], es[i] = 1;
   for (int i = 0; i + 1 < rank; ++i) gs[i] = strides[i];
-  const CUtensorMapSwizzle sw = sw_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+  const CUtensorMapSwizzle sw = sw_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                : sw_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
+                                                 : CU_TENSOR_MAP_SWIZZLE_32B;
   return fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
             CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;

@@ -155,7 +155,7 @@ int idqn_cta_timeline(idqn_handle* h, int slot, unsigned long long* out, int max
 /* CTAs the graph-replayed step gives the Dense_0 update kernel while it runs next to the conv backward chain (0: it runs
  * after the chain on every SM) -- bench.py reports the kernel's in-step bandwidth next to its stand-alone roofline */
 int idqn_dense_update_ctas(idqn_handle* h);
-/* n > 0: that many CTAs; 0: the update runs after the chain on every SM; < 0: automatic (58 + 6.5 K).  Before the first step. */
+/* n > 0: that many CTAs; 0: the update runs after the chain on every SM; < 0: automatic (min(80, 54 + 6 K) on 148 SMs).  Before the first step. */
 int idqn_set_dense_update_ctas(idqn_handle* h, int n);
 /* pipeline timeline of CTA 0 of the kernel named by the IDQN_TL environment variable (fwd0..2, dgrad1..2, wgrad0..2,
  * dfwd3, ddgrad3) during the most recent step: entries (clock64 << 16 | tag), 0 = unused; returns the entry count */
